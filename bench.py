@@ -2,6 +2,7 @@
 """bench.py -- zero-shot variant-scoring throughput of the B200 engine (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model l32] [--batch 256] [--workload snp]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -31,6 +32,13 @@ last step and inside the timed region (the reference-shaped CLI does the same), 
 
 --impl reference times the CPU oracle (the reference's own implementation is not installable offline: its arithmetic lives
 in mamba-ssm / causal-conv1d / HF-hub remote code; DESIGN.md) with all host threads.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path returned in its last step as DIR/<name>.npy (float32 /
+float64; rows of all ranks in rank order, written by rank 0): `logits_acgt` [windows, 4] for the scoring workloads, and for
+--workload long a fixed, seeded sample of rows of the final hidden state (`hidden_sample` [n, 2 * d_model] and its row numbers
+in each rank's flattened [windows * L] state, `hidden_sample_rows`) bounded by DUMP_SAMPLE_BYTES; with --impl reference, the
+CPU oracle's `logits` [windows, L, vocab].  Inputs and weights are seeded, so the same arguments give the same inputs on every
+run and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -58,13 +66,15 @@ MODELS = {"l20": "PlantCaduceus_l20", "l24": "PlantCaduceus_l24", "l28": "PlantC
 TOKEN_IDX = 255
 WINDOW = 512
 LONG = 8192
+DUMP_SAMPLE_BYTES = 32 << 20      # --dump-outputs: float32 bytes of the hidden-state sample of --workload long, all ranks
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 10; 1 for --impl reference --workload long)")
+    ap.add_argument("--warmup", type=int, default=None,
+                    help="untimed steps before them (default 3; 0 for --impl reference --workload long)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--model", default="l32", choices=sorted(MODELS))
     ap.add_argument("--workload", default="snp", choices=["snp", "genome", "mutagenesis", "long"])
@@ -72,12 +82,28 @@ def parse_args():
     ap.add_argument("--genome-bases", type=int, default=200_000_000, help="--workload genome: length of the synthetic chromosome")
     ap.add_argument("--cpu-sample", type=int, default=2, help="windows in the cpu_baseline sample (0 = skip); ~9 s each on 16 cores")
     ap.add_argument("--no-clocks", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     if args.batch is None:
         args.batch = 16 if args.workload == "long" else 256
+    cpu_long = args.impl == "reference" and args.workload == "long"    # one fp32 CPU forward of an 8192-bp window takes minutes
     if args.steps is None:
-        args.steps = 10
+        args.steps = 1 if cpu_long else 10
+    if args.warmup is None:
+        args.warmup = 0 if cpu_long else 3
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     return args
+
+
+def write_dump(out_dir: str, arrays: dict):
+    """arrays: name -> numpy array (float32 / float64), written as out_dir/<name>.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def load_peaks():
@@ -200,8 +226,10 @@ def run_reference(args):
     import torch
     n = 1  # windows per step: the bounded sample
     L = LONG if args.workload == "long" else WINDOW
-    steps, warmup = (min(args.steps, 1), 0) if args.workload == "long" else (args.steps, args.warmup)
-    rate, ms, threads, _ = cpu_oracle_rate(args.model, n, repeats=steps, warmup=warmup, length=L)
+    steps, warmup = args.steps, args.warmup
+    rate, ms, threads, logits = cpu_oracle_rate(args.model, n, repeats=steps, warmup=warmup, length=L)
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, {"logits": logits.float().numpy()})
     per_window = 3 if args.workload == "mutagenesis" else 1     # one masked forward serves the position's 3 alt alleles
     rate *= per_window
     metric, unit = metric_of(args)
@@ -390,9 +418,10 @@ def run_ours(args):
         hidden_host = torch.empty((B, 2 * cfg.d_model), dtype=torch.bfloat16).pin_memory()
         dev_ids = [t.long() for t in dev_ids]
         host_ids64 = [t.cpu().pin_memory() for t in dev_ids]
+        last_hidden = [None]
 
         def step_device(i):
-            model.forward(dev_ids[i % n_batches], output_hidden_states=True, compute_logits=False)
+            last_hidden[0] = model.forward(dev_ids[i % n_batches], output_hidden_states=True, compute_logits=False).hidden_states[-1]
 
         def step_host(i):
             ids = host_ids64[i % n_batches].to(dev, non_blocking=True)
@@ -409,6 +438,24 @@ def run_ours(args):
     launches0 = model.launch_count()
     ms_total = timed(step_device, K, gather=wl != "long")
     per_rank_ms = list(timed.per_rank_ms)
+    if args.dump_outputs:
+        # the last timed step's outputs, taken before the e2e and profiling passes below reuse the buffers
+        extra = {}
+        if wl == "long":
+            rows = B * L
+            n = min(rows, DUMP_SAMPLE_BYTES // (world * 2 * cfg.d_model * 4))
+            sel = np.sort(np.random.default_rng(0).choice(rows, size=n, replace=False))
+            dump = {"hidden_sample": last_hidden[0].reshape(rows, -1)[torch.from_numpy(sel).to(dev)].float()}
+            extra["hidden_sample_rows"] = sel.astype(np.float64)     # the same rows of every rank's batch
+        else:
+            dump = {"logits_acgt": results[K - 1].clone()}
+        if world > 1:      # rows of every rank, in rank order
+            for name, t in dump.items():
+                full = torch.empty((world,) + tuple(t.shape), dtype=t.dtype, device=dev)
+                dist.all_gather_into_tensor(full, t.contiguous())
+                dump[name] = full.reshape((-1,) + tuple(t.shape[1:]))
+        if rank == 0:
+            write_dump(args.dump_outputs, {**{name: t.cpu().numpy() for name, t in dump.items()}, **extra})
     launches = model.launch_count() - launches0
     clocks = sampler.stop() if not args.no_clocks else None
     per_rank_mhz = None
