@@ -524,6 +524,67 @@ int run_mixer_m2(pcad_handle* h, LayerWeights& lw, int S, int L, cudaStream_t st
   return PCAD_OK;
 }
 
+// Mamba-1, low batch / long context: cut every sequence into P concurrent segments while the sequential kernel's grid
+// (E / 64 x S CTAs) would leave resident slots (4 per SM) empty and the segments stay >= 512 steps long.  (Measured:
+// with shorter segments the two extra passes cost more than the parallelism returns -- B = 4, L = 512: 10.9 vs 6.5 ms;
+// and 512-bp windows, the scoring workload, keep the property that a window scores the same bits alone or in a batch.)
+int scan_segments(const pcad_handle* h, int S, int L) {
+  int P = 1;
+  if (!h->time_parallel) return P;
+  const long long ctas = static_cast<long long>((h->E + kScanCH - 1) / kScanCH) * S, slots = 4LL * h->num_sms;
+  while (P < 32 && ctas * P * 2 <= slots && L % (P * 2) == 0 && L / (P * 2) >= 512 &&
+         static_cast<size_t>(S) * P * 2 * 2 * h->E * kScanN * sizeof(float) <= kSegStateBytes)
+    P *= 2;
+  return P;
+}
+
+// ws.xz holds in_proj's output [T, 2E]: x at [0, E), z at [E, 2E).  Leaves y in ws.y.  prune_idx >= 0: the scan may stop once
+// both directions have reached row prune_idx; *pruned tells whether it did (y is then valid only at the rows the head reads).
+int run_mixer_m1(pcad_handle* h, LayerWeights& lw, int S, int L, int prune_idx, bool* pruned, cudaStream_t st) {
+  Workspace& ws = h->ws;
+  const long long T = static_cast<long long>(S) * L;
+  const int E = h->E, R = h->R, RP = h->RP;
+  const bool f32 = h->f32;
+  int rc;
+  {
+    StageTimer tm(h, st, PCAD_ST_CONV);
+    rc = op_conv(h, ws.xz, 2 * E, lw.dir[0].conv_w, lw.dir[0].conv_b, lw.dir[1].conv_w, lw.dir[1].conv_b, ws.xc[0], ws.xc[1], S, L, E, f32, st);
+    if (rc) return rc;
+  }
+  const int P = scan_segments(h, S, L);
+  // dt_proj runs inside the scan kernel (tcgen05, scan.cuh) unless the time-parallel passes need delta in memory
+  const bool fuse_dt = h->fuse_dt && P == 1;
+  for (int dir = 0; dir < 2; ++dir) {
+    {
+      StageTimer tm(h, st, PCAD_ST_X_PROJ);
+      rc = op_linear(h, ws.xc[dir], lw.dir[dir].x_proj, ws.dbc[dir], T, RP, E, E, E, RP, f32, h->num_sms, st);
+      if (rc) return rc;
+    }
+    if (!fuse_dt) {
+      StageTimer tm(h, st, PCAD_ST_DT_PROJ);
+      rc = op_linear(h, ws.dbc[dir], lw.dir[dir].dt_proj, ws.delta[dir], T, E, R, RP, R, E, f32, h->num_sms, st);
+      if (rc) return rc;
+    }
+  }
+  StageTimer tm(h, st, PCAD_ST_SCAN);
+  const uint8_t* zbase = static_cast<const uint8_t*>(ws.xz) + static_cast<size_t>(E) * h->act_size;
+  *pruned = prune_idx >= 0 && P == 1 && L >= 8;
+  const int Lrun = *pruned ? (prune_idx > L - 1 - prune_idx ? prune_idx : L - 1 - prune_idx) + 1 : 0;
+  // fp32 B|C rows + one-barrier scan mode: one more (tiny) launch per layer, so only where the scan is long enough to
+  // repay it (measured: -1 ms of 170 per step at T = 262 144; launch-bound small batches keep the in-kernel conversion)
+  const bool use_bcf = h->bc_f32 && !f32 && (h->bc_f32_force || T >= 65536);
+  if (fuse_dt)   // the scan reads the x_proj outputs (dt | B | C) and the dt_proj weights
+    return op_biscan(h, ws.xc[0], ws.dbc[0], ws.dbc[0], ws.xc[1], ws.dbc[1], ws.dbc[1], RP, R, zbase, 2 * E,
+                     lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32,
+                     st, lw.dir[0].dt_proj, lw.dir[1].dt_proj, R, R, 1, nullptr, nullptr, Lrun);
+  rc = op_biscan(h, ws.xc[0], ws.delta[0], ws.dbc[0], ws.xc[1], ws.delta[1], ws.dbc[1], RP, R, zbase, 2 * E,
+                 lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32, st,
+                 nullptr, nullptr, 0, 0, P, ws.seg_state, ws.seg_sumd, Lrun, use_bcf ? ws.bcf : nullptr);
+  if (P > 1) h->launch_count += 2;
+  if (use_bcf) h->launch_count += 1;
+  return rc;
+}
+
 // Score-only last layer: rows (s, row_s) of a [S*L, width] tensor -> compact [S, width]; row_s = idx for the forward strands
 // (s < B) and L-1-idx for the RC strands.  16-byte vectors.
 __global__ void gather_rows_kernel(const uint4* __restrict__ src, uint4* __restrict__ dst, int S, int B, int L, int idx, int vec_per_row) {
@@ -544,7 +605,7 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
   Workspace& ws = h->ws;
   const long long T = 2LL * B * L;
   const int S = 2 * B;
-  const int d = h->d, E = h->E, R = h->R, RP = h->RP;
+  const int d = h->d, E = h->E;
   const bool f32 = h->f32;
   const bool res_f32 = f32 || h->cfg.residual_in_fp32;
   const bool fused = h->fuse_norm;
@@ -556,6 +617,12 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
   const int parts = gemm_sumsq_parts(d);
   const int n_in = h->m2 ? h->DIP : 2 * E;          // in_proj output width and row pitch
   const long long ld_in = h->m2 ? h->DIPP : 2 * E;
+  // The block tail: out_proj reads `rows` rows of y and writes x (adding the residual stream res in the fused path), the
+  // final norm reads x and res.  All T rows, unless the last layer was pruned to the 2B rows the head reads.
+  long long rows = T;
+  void* y = ws.y;
+  void* res = ws.resid;
+  void* x = fused ? ws.resid : ws.hid;
   {
     StageTimer tm(h, st, PCAD_ST_EMBED, fused ? 2 : 1);
     const long long total = T * (d / 8);
@@ -568,7 +635,6 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
   for (int li = 0; li < h->cfg.n_layer; ++li) {
     LayerWeights& lw = h->layers[li];
     int rc;
-    bool pruned = false;
     if (!fused) {
       StageTimer tm(h, st, PCAD_ST_NORM);
       rc = op_add_rmsnorm(h, ws.hid, li == 0 ? nullptr : ws.resid, lw.norm_w, ws.normed, ws.resid, T, d, h->cfg.norm_eps, f32, res_f32, st);
@@ -588,122 +654,50 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
       }
       if (rc) return rc;
     }
-    if (h->m2) {
-      rc = run_mixer_m2(h, lw, S, L, st);
-      if (rc) return rc;
-    } else {
-    {
-      StageTimer tm(h, st, PCAD_ST_CONV);
-      rc = op_conv(h, ws.xz, 2 * E, lw.dir[0].conv_w, lw.dir[0].conv_b, lw.dir[1].conv_w, lw.dir[1].conv_b, ws.xc[0], ws.xc[1], S, L, E, f32, st);
-      if (rc) return rc;
-    }
-    // low batch / long context: cut every sequence into P concurrent segments while the sequential kernel's grid
-    // (E / 64 x S CTAs) would leave resident slots (4 per SM) empty and the segments stay >= 512 steps long.  (Measured:
-    // with shorter segments the two extra passes cost more than the parallelism returns -- B = 4, L = 512: 10.9 vs 6.5 ms;
-    // and 512-bp windows, the scoring workload, keep the property that a window scores the same bits alone or in a batch.)
-    int P = 1;
-    if (h->time_parallel) {
-      const long long ctas = static_cast<long long>((E + kScanCH - 1) / kScanCH) * S, slots = 4LL * h->num_sms;
-      while (P < 32 && ctas * P * 2 <= slots && L % (P * 2) == 0 && L / (P * 2) >= 512 &&
-             static_cast<size_t>(S) * P * 2 * 2 * E * kScanN * sizeof(float) <= kSegStateBytes)
-        P *= 2;
-    }
-    // dt_proj runs inside the scan kernel (tcgen05, scan.cuh) unless the time-parallel passes need delta in memory
-    const bool fuse_dt = h->fuse_dt && P == 1;
-    for (int dir = 0; dir < 2; ++dir) {
-      {
-        StageTimer tm(h, st, PCAD_ST_X_PROJ);
-        rc = op_linear(h, ws.xc[dir], lw.dir[dir].x_proj, ws.dbc[dir], T, RP, E, E, E, RP, f32, h->num_sms, st);
-        if (rc) return rc;
-      }
-      if (!fuse_dt) {
-        StageTimer tm(h, st, PCAD_ST_DT_PROJ);
-        rc = op_linear(h, ws.dbc[dir], lw.dir[dir].dt_proj, ws.delta[dir], T, E, R, RP, R, E, f32, h->num_sms, st);
-        if (rc) return rc;
-      }
-    }
-    {
-      StageTimer tm(h, st, PCAD_ST_SCAN);
-      const uint8_t* zbase = static_cast<const uint8_t*>(ws.xz) + static_cast<size_t>(E) * h->act_size;
-      pruned = prune_idx >= 0 && li == h->cfg.n_layer - 1 && P == 1 && h->prune_last && L >= 8;
-      const int Lrun = pruned ? (prune_idx > L - 1 - prune_idx ? prune_idx : L - 1 - prune_idx) + 1 : 0;
-      // fp32 B|C rows + one-barrier scan mode: one more (tiny) launch per layer, so only where the scan is long enough to
-      // repay it (measured: -1 ms of 170 per step at T = 262 144; launch-bound small batches keep the in-kernel conversion)
-      const bool use_bcf = h->bc_f32 && !f32 && (h->bc_f32_force || T >= 65536);
-      if (fuse_dt)   // the scan reads the x_proj outputs (dt | B | C) and the dt_proj weights
-        rc = op_biscan(h, ws.xc[0], ws.dbc[0], ws.dbc[0], ws.xc[1], ws.dbc[1], ws.dbc[1], RP, R, zbase, 2 * E,
-                       lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32,
-                       st, lw.dir[0].dt_proj, lw.dir[1].dt_proj, R, R, 1, nullptr, nullptr, Lrun);
-      else {
-        rc = op_biscan(h, ws.xc[0], ws.delta[0], ws.dbc[0], ws.xc[1], ws.delta[1], ws.dbc[1], RP, R, zbase, 2 * E,
-                       lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32, st,
-                       nullptr, nullptr, 0, 0, P, ws.seg_state, ws.seg_sumd, Lrun, use_bcf ? ws.bcf : nullptr);
-        if (P > 1) h->launch_count += 2;
-        if (use_bcf) h->launch_count += 1;
-      }
-      if (rc) return rc;
-    }
-    }   // Mamba-1 mixer
+    bool pruned = false;
+    rc = h->m2 ? run_mixer_m2(h, lw, S, L, st)
+               : run_mixer_m1(h, lw, S, L, li == h->cfg.n_layer - 1 ? prune_idx : -1, &pruned, st);
+    if (rc) return rc;
     if (pruned) {
-      h->last_pruned = true;
-      // compact tail: y and the residual stream at the 2B rows the head reads -> out_proj (+ residual) -> final norm, [2B, d]
+      // compact tail: y and the residual stream at the 2B rows the head reads; out_proj and the final norm then run on those
       const size_t a = h->act_size, rs = res_f32 ? 4 : a;
       uint8_t* yc = static_cast<uint8_t*>(ws.delta[0]);                                  // [S, E]   (delta is dead after the scan)
       uint8_t* rc_in = static_cast<uint8_t*>(ws.delta[1]);                               // [S, d]   residual rows
-      uint8_t* rc_out = rc_in + align_up(static_cast<size_t>(S) * d * 4, 1024);          // [S, d]   new residual / out_proj output
       {
         StageTimer tm(h, st, PCAD_ST_MISC, 2);
         const int vy = static_cast<int>(E * a / 16), vr = static_cast<int>(d * rs / 16);
         gather_rows_kernel<<<static_cast<unsigned>((static_cast<long long>(S) * vy + 255) / 256), 256, 0, st>>>(
             static_cast<const uint4*>(ws.y), reinterpret_cast<uint4*>(yc), S, B, L, prune_idx, vy);
-        if (fused || li > 0)
-          gather_rows_kernel<<<static_cast<unsigned>((static_cast<long long>(S) * vr + 255) / 256), 256, 0, st>>>(
-              static_cast<const uint4*>(ws.resid), reinterpret_cast<uint4*>(rc_in), S, B, L, prune_idx, vr);
+        gather_rows_kernel<<<static_cast<unsigned>((static_cast<long long>(S) * vr + 255) / 256), 256, 0, st>>>(
+            static_cast<const uint4*>(ws.resid), reinterpret_cast<uint4*>(rc_in), S, B, L, prune_idx, vr);
         CUDA_TRY(h, cudaGetLastError());
       }
-      {
-        StageTimer tm(h, st, PCAD_ST_OUT_PROJ);
-        if (fused) {
-          EpiParams ep;
-          ep.resid = reinterpret_cast<const bf16*>(rc_in);
-          ep.ld_res = d;
-          ep.sumsq_out = ws.sumsq[cur ^ 1];
-          ep.sumsq_parts = parts;
-          rc = op_linear(h, yc, lw.out_proj, rc_out, S, d, E, E, E, d, false, h->num_sms, st, kEpiResidual, ep);
-        } else {
-          rc = op_linear(h, yc, lw.out_proj, rc_out, S, d, E, E, E, d, f32, h->num_sms, st);
-        }
-        if (rc) return rc;
-      }
-      StageTimer tm(h, st, PCAD_ST_NORM);
-      if (fused) rc = op_add_rmsnorm(h, rc_out, nullptr, h->norm_f, ws.normed, nullptr, S, d, h->cfg.norm_eps, false, false, st);
-      else rc = op_add_rmsnorm(h, rc_out, li == 0 ? nullptr : rc_in, h->norm_f, ws.normed, nullptr, S, d, h->cfg.norm_eps, f32, res_f32, st);
-      return rc;
+      h->last_pruned = true;
+      rows = S;
+      y = yc;
+      res = rc_in;
+      x = rc_in + align_up(static_cast<size_t>(S) * d * 4, 1024);                       // [S, d]   new residual / out_proj output
     }
     {
       StageTimer tm(h, st, PCAD_ST_OUT_PROJ);
       if (fused) {
         EpiParams ep;
-        ep.resid = static_cast<const bf16*>(ws.resid);
+        ep.resid = static_cast<const bf16*>(res);
         ep.ld_res = d;
         ep.sumsq_out = ws.sumsq[cur ^ 1];
         ep.sumsq_parts = parts;
-        rc = op_linear(h, ws.y, lw.out_proj, ws.resid, T, d, E, E, E, d, false, h->num_sms, st, kEpiResidual, ep);
+        rc = op_linear(h, y, lw.out_proj, x, rows, d, E, E, E, d, false, h->num_sms, st, kEpiResidual, ep);
         cur ^= 1;
       } else {
-        rc = op_linear(h, ws.y, lw.out_proj, ws.hid, T, d, E, E, E, d, f32, h->num_sms, st);
+        rc = op_linear(h, y, lw.out_proj, x, rows, d, E, E, E, d, f32, h->num_sms, st);
       }
       if (rc) return rc;
     }
   }
-  {
-    StageTimer tm(h, st, PCAD_ST_NORM);
-    int rc;
-    if (fused) rc = op_add_rmsnorm(h, ws.resid, nullptr, h->norm_f, ws.normed, nullptr, T, d, h->cfg.norm_eps, false, false, st);
-    else rc = op_add_rmsnorm(h, ws.hid, h->cfg.n_layer == 0 ? nullptr : ws.resid, h->norm_f, ws.normed, nullptr, T, d, h->cfg.norm_eps, f32, res_f32, st);
-    if (rc) return rc;
-  }
-  return PCAD_OK;
+  // the fused path has already added the residual in out_proj's epilogue; without a layer there is no residual yet
+  StageTimer tm(h, st, PCAD_ST_NORM);
+  return op_add_rmsnorm(h, x, fused || h->cfg.n_layer == 0 ? nullptr : res, h->norm_f, ws.normed, nullptr, rows, d, h->cfg.norm_eps,
+                        f32, res_f32, st);
 }
 
 int run_head(pcad_handle* h, int B, int L, const int* pos_dev, int n_pos, float* out, cudaStream_t st) {
@@ -722,12 +716,47 @@ __global__ void fill_int_kernel(int* p, int n, int v) {
   if (i < n) p[i] = v;
 }
 
-int check_call(pcad_handle* h, int B, int L) {
+constexpr int kNoWork = 1;   // begin_call: B, L or the count is 0, the call returns PCAD_OK without computing anything
+
+// Start of every forward entry point: checks the handle and the shape, returns kNoWork for an empty call, then reports
+// `args_msg` unless `args_ok` (the entry's own pointer and count checks) and checks token_idx (the default 0 is in range for
+// every L > 0).  Returns PCAD_OK once the device is selected and the workspace fits B x L.
+int begin_call(pcad_handle* h, int B, int L, int count, bool args_ok, const char* args_msg, int token_idx = 0) {
   if (!h) return PCAD_ERR_INVALID;
   if (!h->finalized) return fail(h, PCAD_ERR_STATE, "pcad_finalize must succeed before a forward call");
   if (B < 0 || L < 0) return fail(h, PCAD_ERR_INVALID, "negative batch or length");
   if (2LL * B > 65535) return fail(h, PCAD_ERR_INVALID, "B=%d too large for one call (max 32767)", B);
+  if (B == 0 || L == 0 || count == 0) return kNoWork;
+  if (!args_ok) return fail(h, PCAD_ERR_INVALID, "%s", args_msg);
+  if (token_idx < 0 || token_idx >= L) return fail(h, PCAD_ERR_INVALID, "token_idx %d outside [0, %d)", token_idx, L);
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  return ensure_workspace(h, B, L);
+}
+
+// ids (u8 [B, L], device) -> ws.ids, checked: ids >= vocab_size would index past the embedding table / complement map.
+// token_idx >= 0 (score_at): also the head positions ws.pos = token_idx and ws.pos0 = 0.
+int stage_ids(pcad_handle* h, const uint8_t* ids_dev, int B, int L, int token_idx, cudaStream_t st) {
+  Workspace& ws = h->ws;
+  StageTimer tm(h, st, PCAD_ST_MISC, token_idx >= 0 ? 3 : 1);
+  const long long n = static_cast<long long>(B) * L;
+  ids_u8_check_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(ids_dev, ws.ids, n, h->V, h->bad_flag);
+  if (token_idx >= 0) {
+    fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos, B, token_idx);
+    fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos0, B, 0);
+  }
+  CUDA_TRY(h, cudaGetLastError());
   return PCAD_OK;
+}
+
+// Backbone + head at token_idx -> out [B, 4]; ws.ids, ws.pos and ws.pos0 are staged.  One scored position, the same in every
+// window: the last layer is computed only at the rows the head reads.
+int score_at(pcad_handle* h, int B, int L, int token_idx, float* out, cudaStream_t st) {
+  Workspace& ws = h->ws;
+  const bool prune = h->prune_last && !h->m2 && h->cfg.n_layer > 0;
+  int rc = run_backbone(h, B, L, st, prune ? token_idx : -1);
+  if (rc) return rc;
+  if (h->last_pruned) return run_head(h, B, 1, ws.pos0, 1, out, st);   // ws.normed is compact [2B, d]
+  return run_head(h, B, L, ws.pos, 1, out, st);
 }
 
 }  // namespace
@@ -1100,11 +1129,7 @@ int score_core(pcad_handle* h, int B, int L, int token_idx, cudaStream_t st) {
     fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos0, B, 0);
     CUDA_TRY(h, cudaGetLastError());
   }
-  const bool prune = h->prune_last && !h->m2 && h->cfg.n_layer > 0;
-  int rc = run_backbone(h, B, L, st, prune ? token_idx : -1);
-  if (rc) return rc;
-  if (prune && h->last_pruned) return run_head(h, B, 1, ws.pos0, 1, ws.logits4, st);   // ws.normed is compact [2B, d]
-  return run_head(h, B, L, ws.pos, 1, ws.logits4, st);
+  return score_at(h, B, L, token_idx, ws.logits4, st);
 }
 
 // The same through a CUDA graph when the forward is small enough to be launch-bound.  First call with a shape: eager (also
@@ -1159,15 +1184,9 @@ int score_core_graphed(pcad_handle* h, int B, int L, int token_idx, cudaStream_t
 }  // namespace
 
 int pcad_score_windows_dev(pcad_handle* h, const uint8_t* ascii_dev, int B, int L, int token_idx, float* logits4_dev, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0) return PCAD_OK;
-  if (!ascii_dev || !logits4_dev) return fail(h, PCAD_ERR_INVALID, "null argument");
-  if (token_idx < 0 || token_idx >= L) return fail(h, PCAD_ERR_INVALID, "token_idx %d outside [0, %d)", token_idx, L);
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, 1, ascii_dev && logits4_dev, "null argument", token_idx);
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
-  if (rc) return rc;
   Workspace& ws = h->ws;
   const size_t n = static_cast<size_t>(B) * L;
   CUDA_TRY(h, cudaMemcpyAsync(ws.ascii, ascii_dev, n, cudaMemcpyDeviceToDevice, st));
@@ -1178,14 +1197,9 @@ int pcad_score_windows_dev(pcad_handle* h, const uint8_t* ascii_dev, int B, int 
 }
 
 int pcad_forward(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* logits_dev, void* hidden_dev, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0) return PCAD_OK;
-  if (!ids_dev) return fail(h, PCAD_ERR_INVALID, "ids_dev is null");
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, 1, ids_dev, "ids_dev is null");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
-  if (rc) return rc;
   {
     StageTimer tm(h, st, PCAD_ST_MISC);
     const long long n = static_cast<long long>(B) * L;
@@ -1210,68 +1224,31 @@ int pcad_forward(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* lo
 }
 
 int pcad_score_masked(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_mask, float* logits4_dev, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0 || n_mask == 0) return PCAD_OK;
-  if (!ids_dev || !pos_dev || !logits4_dev || n_mask < 0) return fail(h, PCAD_ERR_INVALID, "null or negative argument");
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, n_mask, ids_dev && pos_dev && logits4_dev && n_mask >= 0, "null or negative argument");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
+  rc = stage_ids(h, ids_dev, B, L, -1, st);
   if (rc) return rc;
-  {
-    // copy + validate: ids >= vocab_size would index past the embedding table / complement map
-    StageTimer tm(h, st, PCAD_ST_MISC);
-    const long long n = static_cast<long long>(B) * L;
-    ids_u8_check_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(ids_dev, h->ws.ids, n, h->V, h->bad_flag);
-    CUDA_TRY(h, cudaGetLastError());
-  }
   rc = run_backbone(h, B, L, st);
   if (rc) return rc;
   return run_head(h, B, L, pos_dev, n_mask, logits4_dev, st);
 }
 
 int pcad_score_masked_at(pcad_handle* h, const uint8_t* ids_dev, int token_idx, int B, int L, float* logits4_dev, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0) return PCAD_OK;
-  if (!ids_dev || !logits4_dev) return fail(h, PCAD_ERR_INVALID, "null argument");
-  if (token_idx < 0 || token_idx >= L) return fail(h, PCAD_ERR_INVALID, "token_idx %d outside [0, %d)", token_idx, L);
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, 1, ids_dev && logits4_dev, "null argument", token_idx);
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
+  rc = stage_ids(h, ids_dev, B, L, token_idx, st);
   if (rc) return rc;
-  Workspace& ws = h->ws;
-  {
-    StageTimer tm(h, st, PCAD_ST_MISC, 3);
-    const long long n = static_cast<long long>(B) * L;
-    ids_u8_check_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(ids_dev, ws.ids, n, h->V, h->bad_flag);
-    fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos, B, token_idx);
-    fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos0, B, 0);
-    CUDA_TRY(h, cudaGetLastError());
-  }
-  // one scored position, the same in every window: the last layer is computed only at the rows the head reads
-  const bool prune = h->prune_last && !h->m2 && h->cfg.n_layer > 0;
-  rc = run_backbone(h, B, L, st, prune ? token_idx : -1);
-  if (rc) return rc;
-  if (prune && h->last_pruned) return run_head(h, B, 1, ws.pos0, 1, logits4_dev, st);
-  return run_head(h, B, L, ws.pos, 1, logits4_dev, st);
+  return score_at(h, B, L, token_idx, logits4_dev, st);
 }
 
 int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos, void* hidden_dev, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0 || n_pos == 0) return PCAD_OK;
-  if (!ids_dev || !pos_dev || !hidden_dev || n_pos < 0) return fail(h, PCAD_ERR_INVALID, "null or negative argument");
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, n_pos, ids_dev && pos_dev && hidden_dev && n_pos >= 0, "null or negative argument");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
+  rc = stage_ids(h, ids_dev, B, L, -1, st);
   if (rc) return rc;
-  {
-    StageTimer tm(h, st, PCAD_ST_MISC);
-    const long long n = static_cast<long long>(B) * L;
-    ids_u8_check_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(ids_dev, h->ws.ids, n, h->V, h->bad_flag);
-    CUDA_TRY(h, cudaGetLastError());
-  }
   rc = run_backbone(h, B, L, st);
   if (rc) return rc;
   StageTimer tm(h, st, PCAD_ST_MISC);
@@ -1284,15 +1261,9 @@ int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_de
 }
 
 int pcad_score_windows_host(pcad_handle* h, const uint8_t* ascii_host, int B, int L, int token_idx, float* logits4_host, void* stream) {
-  int rc = check_call(h, B, L);
-  if (rc) return rc;
-  if (B == 0 || L == 0) return PCAD_OK;
-  if (!ascii_host || !logits4_host) return fail(h, PCAD_ERR_INVALID, "null argument");
-  if (token_idx < 0 || token_idx >= L) return fail(h, PCAD_ERR_INVALID, "token_idx %d outside [0, %d)", token_idx, L);
-  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = begin_call(h, B, L, 1, ascii_host && logits4_host, "null argument", token_idx);
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_workspace(h, B, L);
-  if (rc) return rc;
   Workspace& ws = h->ws;
   CUDA_TRY(h, cudaMemcpyAsync(ws.ascii, ascii_host, static_cast<size_t>(B) * L, cudaMemcpyHostToDevice, st));
   rc = score_core_graphed(h, B, L, token_idx, st);

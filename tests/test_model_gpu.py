@@ -347,7 +347,9 @@ def test_small_batch_cuda_graph_replay_is_bit_identical(Model, cuda_device, monk
 
 @pytest.mark.parametrize("kw,dtype", [(dict(d_model=256, n_layer=3), torch.bfloat16), (dict(d_model=128, n_layer=1), torch.bfloat16),
                                       (dict(d_model=256, n_layer=2, residual_in_fp32=True), torch.bfloat16),
-                                      (dict(d_model=128, n_layer=2), torch.float32)])
+                                      (dict(d_model=128, n_layer=2), torch.float32),
+                                      (dict(d_model=128, n_layer=1), torch.float32),
+                                      (dict(d_model=128, n_layer=1, residual_in_fp32=True), torch.bfloat16)])
 def test_score_only_last_layer_pruning_is_bit_identical(Model, cuda_device, monkeypatch, kw, dtype):
     """Score-only calls compute the last layer only as far as the head needs it (the scan stops once both directions have reached
     the scored position; out_proj, residual add and final norm run on the 2B rows the head reads).  Same bits as the full
