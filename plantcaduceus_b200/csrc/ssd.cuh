@@ -177,7 +177,8 @@ gated_norm_sum_kernel(const T* __restrict__ y_f, const T* __restrict__ y_r, cons
 // bf16 variant with the gate cached.  The generic kernel above is MUFU-bound in bf16 (ncu: XU pipe 82 %: SiLU = ex2 + rcp per
 // element, evaluated in both passes) while its second pass already hits L2 (DRAM reads = one pass).  Here SiLU(z) is evaluated
 // once and parked as fp16 in registers (CH 16-byte vectors per lane, E <= 256 CH; 2^-11 relative, below the bf16 rounding of
-// the output; the statistics use the un-rounded fp32 value); y_f / y_r are re-read in the second pass (L2).  Keeping all
+// the output, down to |SiLU(z)| = 2^-14; below that fp16 is subnormal and the gate is exact only to 2^-25 absolute, which is
+// 2^-25 of |y| rstd |w| on such an element; the statistics use the un-rounded fp32 value); y_f / y_r are re-read in the second pass (L2).  Keeping all
 // three tensors in registers instead (one DRAM/L2 pass, 126-230 registers) measured slower: 1.0 vs 0.71 ms per layer at
 // E = 1536 -- too few warps left to overlap the loads with the arithmetic.
 template <int CH>
