@@ -221,6 +221,25 @@ int pcad_op_biscan_segmented(const void* u_f, const void* delta_f, const void* b
                              void* y, int S, int L, int E, int segments, float* seg_state, float* seg_sumd,
                              int dtype, void* stream);
 
+/* pcad_op_biscan with the scan modes the forward picks for itself, for testing them one operator at a time (the forward
+ * runs the same host function):
+ *   segments <= 1:  the sequential scan.  segments >= 2: time-parallel, as pcad_op_biscan_segmented (same scratch).
+ *   bc_rows NULL:   B|C are converted to fp32 inside the scan kernel.  Otherwise (bf16 only) float [2][S*L][32] scratch:
+ *                   rows [B ln 2 | C] of the forward direction, then of the reverse direction, written by a conversion
+ *                   kernel before the scan, which then reads them by TMA.  What the bf16 forward runs at S*L >= 65536.
+ *   Lrun 0 or L:    every row of y holds its final value.  (L+1)/2 <= Lrun < L (sequential only): each direction stops
+ *                   after Lrun steps, as the forward's score-only last layer does; only rows [L-Lrun, Lrun) of every
+ *                   sequence hold final values, the other rows hold one direction's parked partial.
+ * Returns PCAD_ERR_INVALID, before launching anything, for bc_rows with fp32, Lrun < 0, Lrun > L, 0 < Lrun < (L+1)/2
+ * (some rows would be visited by neither direction), and Lrun < L with segments >= 2. */
+int pcad_op_biscan_ex(const void* u_f, const void* delta_f, const void* bc_f,
+                      const void* u_r, const void* delta_r, const void* bc_r,
+                      int64_t ldbc, int bc_off, const void* z, int64_t ldz,
+                      const float* A_f, const float* D_f, const float* dt_bias_f,
+                      const float* A_r, const float* D_r, const float* dt_bias_r,
+                      void* y, int S, int L, int E, int segments, float* seg_state, float* seg_sumd,
+                      float* bc_rows, int Lrun, int dtype, void* stream);
+
 /* The same with Mamba.dt_proj [F.linear(dt, dt_proj.weight)] computed inside the scan kernel on the tensor core (bf16 only):
  * dbc_* are the x_proj outputs [S*L, ldbc] (dt in columns [0, R), B at [bc_off, bc_off+16), C at [bc_off+16, bc_off+32);
  * ldbc >= 64), wdt_* the dt_proj weights [E, R] with row pitch ldw (elements, a multiple of 8; R <= 64).  Delta is rounded

@@ -23,7 +23,8 @@ EXPORTS = (
     "pcad_set_tokenizer", "pcad_take_id_error", "pcad_hidden_at", "pcad_forward", "pcad_score_masked", "pcad_score_masked_at", "pcad_score_windows_host", "pcad_score_windows_dev", "pcad_extract_windows", "pcad_tokenize",
     "pcad_workspace_bytes", "pcad_set_profiling", "pcad_get_profile", "pcad_launch_count",
     "pcad_op_linear", "pcad_op_linear_residual", "pcad_op_linear_rowscale", "pcad_op_sumsq_parts",
-    "pcad_op_add_rmsnorm", "pcad_op_conv_silu", "pcad_op_biscan", "pcad_op_biscan_segmented", "pcad_op_biscan_dt",
+    "pcad_op_add_rmsnorm", "pcad_op_conv_silu", "pcad_op_biscan", "pcad_op_biscan_segmented", "pcad_op_biscan_ex",
+    "pcad_op_biscan_dt",
     "pcad_op_ssd_scan", "pcad_op_gated_norm_sum",
 )
 
@@ -90,6 +91,8 @@ def load() -> C.CDLL:
                                    i32, i32, i32, i32, vp]
     lib.pcad_op_biscan_segmented.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp,
                                              i32, i32, i32, i32, vp, vp, i32, vp]
+    lib.pcad_op_biscan_ex.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp,
+                                      i32, i32, i32, i32, vp, vp, vp, i32, i32, vp]
     lib.pcad_op_ssd_scan.argtypes = [vp, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
     lib.pcad_op_gated_norm_sum.argtypes = [vp, vp, vp, i64, vp, vp, vp, i64, i32, C.c_float, i32, vp]
     for name in EXPORTS:

@@ -332,6 +332,14 @@ int op_biscan(pcad_handle* h, const void* u_f, const void* delta_f, const void* 
     return fail(h, PCAD_ERR_INVALID, "biscan: E, ldbc, bc_off, ldz must be multiples of %d elements", vec);
   if (S <= 0 || L <= 0) return PCAD_OK;
   if (S > 65535) return fail(h, PCAD_ERR_INVALID, "biscan: at most 65535 sequences per call");
+  // rejected before anything is launched: these combinations used to be accepted with one argument silently ignored
+  if (bcf && (f32 || wdt_f || wdt_r))
+    return fail(h, PCAD_ERR_INVALID, "biscan: fp32 B|C rows are a mode of the bf16 scan without the in-kernel dt_proj");
+  if (Lrun < 0 || Lrun > L || (Lrun > 0 && Lrun < (L + 1) / 2))
+    return fail(h, PCAD_ERR_INVALID, "biscan: Lrun = %d must be 0 or in [(L+1)/2, L] = [%d, %d] (below, some rows are visited by neither direction)",
+                Lrun, (L + 1) / 2, L);
+  if (Lrun > 0 && Lrun < L && segments > 1)
+    return fail(h, PCAD_ERR_INVALID, "biscan: an early-stopped scan (Lrun < L) cannot be time-parallel (segments > 1)");
   cudaError_t e;
 #define PCAD_SCAN_ARGS(TT)                                                                                           \
   static_cast<const TT*>(u_f), static_cast<const TT*>(delta_f), static_cast<const TT*>(bc_f), static_cast<const TT*>(u_r), \
@@ -1395,6 +1403,16 @@ int pcad_op_biscan_segmented(const void* u_f, const void* delta_f, const void* b
   return op_fail_to_global(op_biscan(op_scratch(), u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, dt_bias_f,
                                      A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream), nullptr,
                                      nullptr, 0, 0, segments, seg_state, seg_sumd));
+}
+
+int pcad_op_biscan_ex(const void* u_f, const void* delta_f, const void* bc_f, const void* u_r, const void* delta_r, const void* bc_r,
+                      int64_t ldbc, int bc_off, const void* z, int64_t ldz, const float* A_f, const float* D_f, const float* dt_bias_f,
+                      const float* A_r, const float* D_r, const float* dt_bias_r, void* y, int S, int L, int E, int segments,
+                      float* seg_state, float* seg_sumd, float* bc_rows, int Lrun, int dtype, void* stream) {
+  if (dtype != PCAD_BF16 && dtype != PCAD_F32) return PCAD_ERR_INVALID;
+  return op_fail_to_global(op_biscan(op_scratch(), u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, dt_bias_f,
+                                     A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream), nullptr,
+                                     nullptr, 0, 0, segments < 1 ? 1 : segments, seg_state, seg_sumd, Lrun, bc_rows));
 }
 
 int pcad_op_ssd_scan(const void* xbc_f, const void* xbc_r, int64_t ld_xbc, const void* dt_raw, int64_t ld_dt, const float* A_f,

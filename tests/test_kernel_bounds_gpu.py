@@ -51,6 +51,9 @@ K = {
     "scan_bf16": 1.25, "scan_f32": 0.375, "segscan_bf16": 1.25, "segscan_f32": 0.45,
     "softplus_bf16": 1.5, "softplus_f32": 12.0, "decay_bf16": 1.5, "decay_f32": 4.0,
     "ssd_tc": 1.3, "ssd_seq_bf16": 1.0, "ssd_seq_f32": 0.7, "gnorm_bf16": 2.0, "gnorm_f32": 0.2,
+    "head": 4e-4,     # measured maximum 1.85e-4 (fp32, PlantCaduceus_l32 widths, B = 256, L = 512)
+
+    "bc_rows": 1.0,   # a priori, not measured: one rounding of the product and one of ln 2 (2^-24 |ref| each) bound it by 1
 }
 
 PLANTCADUCEUS = ["PlantCaduceus_l20", "PlantCaduceus_l24", "PlantCaduceus_l28", "PlantCaduceus_l32"]
@@ -655,12 +658,18 @@ def scan_units(dtype):
     return (U_OUT[BF16], 2.0 ** -8) if dtype == BF16 else (U32, 2 * NS * U32)
 
 
+def scan_args(si, y):
+    """The 20 data arguments every pcad_op_biscan* entry point starts with."""
+    E = si.E
+    return (vp(si.u[0]), vp(si.dl[0]), vp(si.bc[0]), vp(si.u[1]), vp(si.dl[1]), vp(si.bc[1]), si.RP, si.R, vp(si.xz, E), 2 * E,
+            vp(si.A[0]), vp(si.D[0]), vp(si.bias[0]), vp(si.A[1]), vp(si.D[1]), vp(si.bias[1]), y.ptr, si.S, si.L, E)
+
+
 def run_biscan(lib, si, segments=0):
     S, L, E = si.S, si.L, si.E
     td = TD[si.dtype]
     y = Guarded(S * L, E, td)
-    args = (vp(si.u[0]), vp(si.dl[0]), vp(si.bc[0]), vp(si.u[1]), vp(si.dl[1]), vp(si.bc[1]), si.RP, si.R, vp(si.xz, E), 2 * E,
-            vp(si.A[0]), vp(si.D[0]), vp(si.bias[0]), vp(si.A[1]), vp(si.D[1]), vp(si.bias[1]), y.ptr, S, L, E)
+    args = scan_args(si, y)
     if segments:
         state = Guarded(S * segments * 2 * E, NS, torch.float32)
         sumd = Guarded(S * segments * 2, E, torch.float32)
@@ -692,8 +701,8 @@ def scan_stats(y, si, seqs):
 def test_biscan_matches_float64(lib, dtype, S, E, R):
     """The sequential scan at the scoring batch (S = 512 strands of 512 bp: blockIdx.y up to 511, every channel block); the
     reference covers the first, the last and six random sequences, all channels.  pcad_op_biscan runs the kScanPlain mode
-    (B|C converted in the kernel); the forward at T >= 65536 runs kScanBcF32 (B|C as fp32 rows from bc_to_f32_kernel), which
-    no operator entry point exposes, so that mode is checked only through the model tests."""
+    (B|C converted in the kernel); the mode the bf16 forward runs at T >= 65536 (kScanBcF32: B|C as fp32 rows from
+    bc_to_f32_kernel) is checked on the same inputs by test_biscan_bc_rows_matches_plain_and_float64."""
     si = scan_inputs(S, 512, E, R, dtype, seed=E + S)
     y = run_biscan(lib, si)
     seqs = sample_sequences(S, seed=E)
@@ -709,6 +718,209 @@ def test_biscan_segmented_matches_float64(lib, P, dtype):
     y = run_biscan(lib, si, segments=P)
     st, _, _ = scan_stats(y, si, list(range(S)))
     verdict("segscan_f32" if dtype == F32 else "segscan_bf16", f"P={P} S={S} L={L} E={E}", ("y", st))
+
+
+# ---- the scan as the forward runs it: fp32 B|C rows, time-parallel segments, early stop (pcad_op_biscan_ex) --------------
+SEG_STATE_BYTES = 16 << 20   # kSegStateBytes (csrc/pcad.cu)
+
+
+def scan_segments(E, S, L, num_sms):
+    """Segments per sequence of the forward's Mamba-1 scan (a copy of scan_segments in csrc/pcad.cu, 64-channel CTAs, 4
+    resident per SM)."""
+    P = 1
+    ctas, slots = -(-E // 64) * S, 4 * num_sms
+    while (P < 32 and ctas * P * 2 <= slots and L % (P * 2) == 0 and L // (P * 2) >= 512
+           and S * P * 2 * 2 * E * NS * 4 <= SEG_STATE_BYTES):
+        P *= 2
+    return P
+
+
+def forward_lrun(L, p, P=1):
+    """Steps per direction of the score-only last layer's scan at scored position p (a copy of the line in run_mixer_m1,
+    csrc/pcad.cu); 0: the whole sequence.  Rows [L - Lrun, Lrun) then hold final values."""
+    pruned = p >= 0 and P == 1 and L >= 8
+    return (p if p > L - 1 - p else L - 1 - p) + 1 if pruned else 0
+
+
+def num_sms():
+    return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+
+
+def run_biscan_ex(lib, si, segments=0, bc_rows=False, Lrun=0):
+    """pcad_op_biscan_ex with every buffer it writes (y, the fp32 B|C rows, the segment state) Guarded: (rc, {name: buf})."""
+    S, L, E = si.S, si.L, si.E
+    bufs = {"y": Guarded(S * L, E, TD[si.dtype])}
+    if segments > 1:
+        bufs["seg_state"] = Guarded(S * segments * 2 * E, NS, torch.float32)
+        bufs["seg_sumd"] = Guarded(S * segments * 2, E, torch.float32)
+    if bc_rows:
+        bufs["bc_rows"] = Guarded(2 * S * L, 2 * NS, torch.float32)
+
+    def ptr(k):
+        return bufs[k].ptr if k in bufs else None
+    rc = lib.pcad_op_biscan_ex(*scan_args(si, bufs["y"]), segments, ptr("seg_state"), ptr("seg_sumd"), ptr("bc_rows"), Lrun,
+                               si.dtype, stream())
+    torch.cuda.synchronize()
+    return rc, bufs
+
+
+def run_biscan_ex_ok(lib, si, **kw):
+    rc, bufs = run_biscan_ex(lib, si, **kw)
+    ok(lib, rc)
+    assert_guards(f"biscan_ex {kw}", **bufs)
+    return bufs
+
+
+def untouched(g):
+    return bool((g.raw.view(torch.int16) == SENTINEL).all())
+
+
+def bc_rows_stats(rows, si):
+    """The fp32 B|C scratch: [B ln 2 | C] of both directions.  Bit-exact against the same fp32 product in torch, and within
+    one rounding of the product plus one of ln 2 (2^-24 |ref| each) of float64 on the bf16 inputs."""
+    S, L, R = si.S, si.L, si.R
+    got = rows.t.view(2, S * L, 2 * NS)
+    st = Stats()
+    for k in range(2):
+        bc = si.bc[k][:, R:R + 2 * NS].float()
+        want32 = torch.cat((bc[:, :NS] * torch.tensor(math.log(2.0), dtype=torch.float32, device=DEV), bc[:, NS:]), dim=1)
+        assert torch.equal(got[k], want32), f"B|C rows, direction {k}: not the fp32 product"
+        ref = bc.double() * torch.tensor([math.log(2.0)] * NS + [1.0] * NS, dtype=torch.float64, device=DEV)
+        st.add(got[k], ref, ref.abs(), U32, U32)
+    return st
+
+
+@pytest.mark.parametrize("E,R", [(2048, 64), (768, 24)], ids=["l32", "l20"])
+def test_biscan_bc_rows_matches_plain_and_float64(lib, E, R):
+    """The scan the bf16 forward runs at T >= 65536 (every scan of bench.py): B|C as fp32 rows written by bc_to_f32_kernel and
+    read by TMA (kScanBcF32: its own stage layout, double-buffered ys, one barrier per chunk), at the scoring batch, on the
+    inputs of test_biscan_matches_float64.  Same arithmetic in the same order as kScanPlain: bit-identical output."""
+    S, L = 512, 512
+    si = scan_inputs(S, L, E, R, BF16, seed=E + S)
+    plain = run_biscan(lib, si)
+    bufs = run_biscan_ex_ok(lib, si, bc_rows=True)
+    y = bufs["y"]
+    assert torch.equal(y.t, plain.t), "fp32 B|C rows mode differs from the plain mode"
+    del plain
+    seqs = sample_sequences(S, seed=E)
+    st, _, _ = scan_stats(y, si, seqs)
+    verdict("scan_bf16", f"bc_rows S={S} L={L} E={E} R={R} seqs {seqs}", ("y", st))
+    verdict("bc_rows", f"S={S} L={L} R={R} both directions", ("bc_rows", bc_rows_stats(bufs["bc_rows"], si)))
+
+
+def test_biscan_time_parallel_bc_rows_matches_float64(lib):
+    """Low-batch long context as the forward runs it: B = 1, L = 32768 windows of PlantCaduceus_l20 (S = 2, E = 768,
+    T = 65536: fp32 B|C rows), cut into the number of segments the forward picks on this device (16 on a 148-SM B200)."""
+    S, L, E, R = 2, 32768, 768, 24
+    P = scan_segments(E, S, L, num_sms())
+    assert P > 1 and forward_lrun(L, L // 2, P) == 0
+    si = scan_inputs(S, L, E, R, BF16, seed=321)
+    plain = run_biscan(lib, si, segments=P)
+    y = run_biscan_ex_ok(lib, si, segments=P, bc_rows=True)["y"]
+    assert torch.equal(y.t, plain.t), "time-parallel scan: fp32 B|C rows mode differs from the plain mode"
+    del plain
+    t0 = time.time()
+    st, _, _ = scan_stats(y, si, list(range(S)))
+    verdict("segscan_bf16", f"bc_rows P={P} S={S} L={L} E={E} (float64 reference {time.time() - t0:.1f} s)", ("y", st))
+
+
+SCAN_MODES = [(BF16, False), (BF16, True), (F32, False)]
+SCAN_MODE_IDS = ["bf16", "bf16-bc_rows", "f32"]
+
+
+def check_early_stop(lib, si, full, ref, mag, seqs, p, bc_rows, label):
+    """One early-stopped scan against the full-length run of the same mode (bit-identical on the rows that hold final values)
+    and against float64 there."""
+    S, L, E = si.S, si.L, si.E
+    Lrun = forward_lrun(L, p)
+    assert Lrun > 0
+    y = run_biscan_ex_ok(lib, si, bc_rows=bc_rows, Lrun=Lrun)["y"]
+    lo, hi = L - Lrun, Lrun
+    got = y.t.view(S, L, E)[:, lo:hi]
+    assert torch.equal(got, full.t.view(S, L, E)[:, lo:hi]), f"{label} p={p} Lrun={Lrun}: rows [{lo}, {hi}) differ from the full run"
+    sel = torch.tensor(seqs, device=DEV)
+    u_out, u_acc = scan_units(si.dtype)
+    st = Stats().add(got[sel].reshape(-1, E), ref.view(len(seqs), L, E)[:, lo:hi].reshape(-1, E),
+                     mag.view(len(seqs), L, E)[:, lo:hi].reshape(-1, E), u_out, u_acc)
+    verdict("scan_f32" if si.dtype == F32 else "scan_bf16", f"{label} p={p} Lrun={Lrun} rows [{lo}, {hi})", ("y", st))
+
+
+@pytest.mark.parametrize("dtype,bc_rows", SCAN_MODES, ids=SCAN_MODE_IDS)
+def test_biscan_early_stop_at_the_scoring_batch(lib, dtype, bc_rows):
+    """The score-only last layer (pcad_score_masked_at, the score-window calls, bench.py's scoring workload): each direction
+    stops after max(p, L-1-p) + 1 steps.  l32 widths at the scoring batch, p = 255 (the benchmark's), 256, 100, and 0 (a full
+    run).  bf16 with fp32 B|C rows is exactly the benchmark's last layer."""
+    S, L, E, R = 512, 512, 2048, 64
+    si = scan_inputs(S, L, E, R, dtype, seed=77 + dtype)
+    full = run_biscan_ex_ok(lib, si, bc_rows=bc_rows)["y"]
+    seqs = sample_sequences(S, seed=78)
+    st, ref, mag = scan_stats(full, si, seqs)
+    label = f"early stop {SCAN_MODE_IDS[SCAN_MODES.index((dtype, bc_rows))]} S={S} L={L} E={E}"
+    verdict("scan_f32" if dtype == F32 else "scan_bf16", f"{label} full", ("y", st))
+    for p in (255, 256, 100, 0):
+        check_early_stop(lib, si, full, ref, mag, seqs, p, bc_rows, label)
+
+
+RAGGED_STOPS = [(301, 150), (301, 7), (33, 16), (8, 3), (17, 8)]
+
+
+@pytest.mark.parametrize("dtype,bc_rows", SCAN_MODES, ids=SCAN_MODE_IDS)
+def test_biscan_early_stop_ragged(lib, dtype, bc_rows):
+    """Early stop where the last chunk is partial (nsteps < 16) and the epilogue's has_final / late_chunk paths change:
+    (301, 150) leaves one valid row, (8, 3) is the shortest window the forward prunes (one chunk)."""
+    S, E, R = 6, 512, 32
+    for L, p in RAGGED_STOPS:
+        si = scan_inputs(S, L, E, R, dtype, seed=L * 1000 + p)
+        full = run_biscan_ex_ok(lib, si, bc_rows=bc_rows)["y"]
+        seqs = list(range(S))
+        ref, mag = biscan_reference(si, seqs)
+        label = f"early stop {SCAN_MODE_IDS[SCAN_MODES.index((dtype, bc_rows))]} S={S} L={L} E={E}"
+        check_early_stop(lib, si, full, ref, mag, seqs, p, bc_rows, label)
+
+
+def test_biscan_ex_rejects_bad_arguments(lib):
+    """Combinations pcad_op_biscan_ex refuses: an error code and not one byte of any buffer written."""
+    S, L, E, R = 4, 64, 512, 32
+    sis = {dt: scan_inputs(S, L, E, R, dt, seed=9) for dt in (BF16, F32)}
+    bad = [(F32, 0, True, 0, "fp32 B|C rows"), (F32, 0, True, L, "fp32 B|C rows"),
+           (BF16, 2, False, L - 8, "early stop + time-parallel"), (BF16, 2, True, L // 2, "early stop + time-parallel"),
+           (BF16, 0, False, -1, "Lrun < 0"), (BF16, 0, True, L + 1, "Lrun > L"),
+           (BF16, 0, False, L // 2 - 1, "Lrun < (L+1)/2"), (F32, 0, False, 1, "Lrun < (L+1)/2")]
+    for dtype, segments, bc_rows, Lrun, why in bad:
+        rc, bufs = run_biscan_ex(lib, sis[dtype], segments=segments, bc_rows=bc_rows, Lrun=Lrun)
+        assert rc != 0, f"{why}: accepted (dtype {dtype}, segments {segments}, bc_rows {bc_rows}, Lrun {Lrun})"
+        assert lib.pcad_last_error(None), why
+        assert all(untouched(b) for b in bufs.values()), f"{why}: rejected, but a buffer was written"
+    # the boundaries themselves are accepted: Lrun = (L+1)/2 (odd L), and Lrun = L with time-parallel segments
+    si = scan_inputs(S, 63, E, R, BF16, seed=10)
+    run_biscan_ex_ok(lib, si, bc_rows=True, Lrun=32)
+    run_biscan_ex_ok(lib, sis[BF16], segments=2, bc_rows=True, Lrun=L)
+    print(f"[bounds] biscan_ex: {len(bad)} argument combinations rejected with nothing written; boundaries accepted")
+
+
+def test_scan_mode_choices_match_hand_derived_values():
+    """Needs no device: the Python copies of the forward's scan_segments and Lrun against values worked out by hand."""
+    # l20 (E = 768): B = 1, L = 32768 -> 24 CTAs per segment, 24 * 16 = 384 <= 592 slots, 24 * 32 > 592 -> P = 16
+    assert scan_segments(768, 2, 32768, 148) == 16
+    assert scan_segments(768, 4, 16384, 148) == 8
+    assert scan_segments(768, 2, 8192, 148) == 16       # segments of 512 steps, the shortest allowed
+    assert scan_segments(768, 2, 1000, 148) == 1        # 500-step segments: too short
+    assert scan_segments(768, 2, 2050, 148) == 2        # L / 4 is not an integer
+    assert scan_segments(2048, 512, 512, 148) == 1      # bench.py snp: the grid already fills the GPU
+    assert scan_segments(2048, 32, 8192, 148) == 1      # bench.py long (B = 16): 1024 CTAs
+    assert scan_segments(2048, 2, 65536, 148) == 8
+    assert scan_segments(2048, 2, 65536, 8) == 1
+    # Lrun = max(p, L-1-p) + 1; valid rows [L - Lrun, Lrun)
+    want = {(512, 255): 257, (512, 256): 257, (512, 100): 412, (512, 0): 512, (512, 511): 512,
+            (301, 150): 151, (301, 7): 294, (33, 16): 17, (8, 3): 5, (8, 4): 5, (17, 8): 9}
+    for (L, p), lrun in want.items():
+        assert forward_lrun(L, p) == lrun, (L, p)
+        assert (L + 1) // 2 <= lrun <= L
+        assert L - lrun <= p < lrun                    # the scored row is a valid row
+    assert (301 - forward_lrun(301, 150), forward_lrun(301, 150)) == (150, 151)   # exactly one valid row
+    assert forward_lrun(7, 3) == 0                     # windows shorter than 8 are not pruned
+    assert forward_lrun(512, 255, P=2) == 0            # nor is a time-parallel scan
+    assert forward_lrun(512, -1) == 0
 
 
 def unit_scan_inputs(S, L, E, dtype, R=8):
@@ -886,6 +1098,94 @@ def test_gated_norm_sum_matches_float64(lib, E, dtype):
     verdict("gnorm_f32" if dtype == F32 else "gnorm_bf16", f"rows={rows} E={E} ldz={DIPP}", ("out", st))
 
 
+# ---- embedding, final norm, RC LM head and hidden taps (a model without layers) -----------------------------------------
+EMB_KEY = "caduceus.backbone.embeddings.word_embeddings.embedding.weight"
+HEAD_KEY = "lm_head.lm_head.weight"
+NORM_KEY = "caduceus.backbone.norm_f.weight"
+HEAD_ROWS = 8192   # rows per float64 chunk
+
+
+def bf16_exact(t):
+    return t.to(torch.bfloat16).float()
+
+
+@pytest.mark.parametrize("dtype", [BF16, F32], ids=["bf16", "f32"])
+@pytest.mark.parametrize("B,L", [(256, 512), (16, 8192)], ids=["snp", "long"])
+@pytest.mark.parametrize("name", LARGEST)
+def test_embedding_norm_and_rc_head_match_float64(cuda_device, name, B, L, dtype):
+    """embed -> final norm -> RC LM head at the benchmark shapes, through the model with n_layer = 0, so every output is the
+    engine's: hidden_states[-1] = [RMSNorm(emb[id]) w | flip_channels(RMSNorm(emb[comp[id]]) w)] against float64 (the RC half
+    carries the complement map, the sequence flip and the channel flip), the logits against float64 of the RC head applied to
+    the engine's own hidden output, and every scoring / tap entry point against the matching slice, bit for bit.  Weights are
+    bf16-representable, so both dtypes see the same numbers; the ids cover all eight (PAD, mask, N, a, c, g, t, 7)."""
+    from plantcaduceus_b200.modeling import CaduceusForMaskedLM
+    from plantcaduceus_b200.tokenizer import CharDNATokenizer
+    import dataclasses
+    import numpy as np
+    cfg = dataclasses.replace(preset(name), n_layer=0)
+    d, V = cfg.d_model, cfg.vocab_size
+    g = torch.Generator().manual_seed(d + L + dtype)
+    sd = {EMB_KEY: bf16_exact(torch.randn(V, d, generator=g) * torch.exp(torch.randn(V, 1, generator=g))),
+          HEAD_KEY: bf16_exact(torch.randn(V, d, generator=g) * d ** -0.5),
+          NORM_KEY: bf16_exact(torch.randn(d, generator=g) * 0.3 + 1.0)}
+    model = CaduceusForMaskedLM.from_pretrained(sd, config=cfg, torch_dtype=TD[dtype]).to(cuda_device)
+    tok = CharDNATokenizer()
+    acgt = [tok.get_vocab()[c] for c in "acgt"]
+    # ASCII windows with upper- and lower-case bases and N, masked at token_idx as the score-window calls mask them; then
+    # PAD and id 7 (which no byte maps to) at a few other positions.  Without a layer every position's outputs depend on its
+    # own id only, so the score-window calls still see the same inputs at token_idx.
+    token_idx = L // 2 - 1
+    ascii_ = torch.tensor(list(b"ACGTNacgtn"), dtype=torch.uint8)[torch.randint(0, 10, (B, L), generator=g)]
+    lut = torch.as_tensor(np.asarray(tok.lut, dtype=np.uint8))
+    ids = lut[ascii_.long()].clone()
+    ids[:, token_idx] = tok.mask_token_id
+    ids.view(-1)[torch.randperm(B * L, generator=g)[:B * L // 16]] = torch.tensor([0, 7], dtype=torch.uint8).repeat(B * L // 32)
+    ids[:, token_idx] = tok.mask_token_id
+    assert set(ids.unique().tolist()) == set(range(V))
+    ids_dev = ids.to(cuda_device)
+    out = model(input_ids=ids_dev.long(), output_hidden_states=True)
+    logits, hid = out.logits, out.hidden_states[-1]
+    assert logits.shape == (B, L, V) and hid.shape == (B, L, 2 * d)
+    # float64 reference rows, one per id: RMSNorm(emb[v]) w, and the RC half flip_channels(RMSNorm(emb[comp[v]]) w)
+    comp = torch.tensor([cfg.complement_map.get(i, i) for i in range(V)], device=DEV)
+    emb = sd[EMB_KEY].double().to(DEV)
+    normed = emb * torch.rsqrt(emb.pow(2).mean(-1, keepdim=True) + cfg.norm_epsilon) * sd[NORM_KEY].double().to(DEV)
+    table = torch.cat((normed, normed[comp].flip(-1)), dim=1)                        # [V, 2d]
+    W = sd[HEAD_KEY].double().to(DEV)
+    Wc = W[comp]
+    ids_flat, hid_flat, lg_flat = ids_dev.view(-1).long(), hid.view(B * L, 2 * d), logits.view(B * L, V)
+    sh, sl = Stats(), Stats()
+    for r0 in range(0, B * L, HEAD_ROWS):
+        r1 = min(B * L, r0 + HEAD_ROWS)
+        ref = table[ids_flat[r0:r1]]
+        sh.add(hid_flat[r0:r1], ref, ref.abs(), U_OUT[dtype], U32 * d, row0=r0)
+        hf, hr = hid_flat[r0:r1, :d].double(), hid_flat[r0:r1, d:].flip(-1).double()
+        ref = hf @ W.t() + hr @ Wc.t()
+        mag = hf.abs() @ W.abs().t() + hr.abs() @ Wc.abs().t()
+        sl.add(lg_flat[r0:r1], ref, mag, U32, U32 * 2 * d, row0=r0)
+        del ref, mag, hf, hr
+    case = f"{name} n_layer=0 B={B} L={L} {TD[dtype]}"
+    verdict("norm_f32" if dtype == F32 else "norm_bf16", case, ("hidden", sh))
+    verdict("head", case, ("logits", sl))
+    # the entry points against slices of the full outputs
+    b_idx = torch.arange(B, device=DEV)[:, None]
+    pos = torch.randint(0, L, (B, 5), generator=g).to(DEV, torch.int32)
+    pos[:, 0], pos[:, 1], pos[:, 2] = 0, L - 1, token_idx
+    acgt_dev = torch.tensor(acgt, device=DEV)
+    want4 = logits[:, token_idx][:, acgt_dev]
+    checks = {
+        "hidden_at": (model.hidden_at(ids_dev, pos), hid[b_idx, pos.long()]),
+        "score_masked": (model.score_masked(ids_dev, pos), logits[b_idx, pos.long()][..., acgt_dev]),
+        "score_masked_at": (model.score_masked(ids_dev, token_idx)[:, 0], want4),
+        "score_windows_host": (model.score_windows_host(ascii_.numpy(), token_idx).to(DEV), want4),
+        "score_windows_device": (model.score_windows_device(ascii_.to(cuda_device), token_idx), want4),
+    }
+    torch.cuda.synchronize()
+    bad = [k for k, (got, want) in checks.items() if not torch.equal(got, want)]
+    print(f"[bounds] {'entry points':14s} {case}: {', '.join(checks)} bit-identical to the full outputs: {not bad}")
+    assert not bad, f"{case}: {bad} differ from the matching slice of the full forward"
+
+
 # ---- the checkers can fail ---------------------------------------------------------------------------------------------
 def test_checkers_reject_wrong_outputs(lib):
     """Each checker above, fed a copy of a real kernel output with one deliberate error, rejects it.  CPU-side edits of
@@ -940,3 +1240,13 @@ def test_checkers_reject_wrong_outputs(lib):
     sb = Stats().add(bad.to(torch.bfloat16).view(-1, 768), ref, mag, u_out, u_acc)
     print(f"[bounds] self-check scan: 2^-5 D u SiLU(z) on one channel -> max err/unit {sb.ratio:.4g} (k = {K['scan_bf16']})")
     assert rejects("scan_bf16", sb)
+    # early stop one step short of the forward's Lrun at p = 255: a legal call whose valid rows [256, 256) are empty; row 255
+    # keeps the forward direction's parked partial.  The checker must pass row 255 at Lrun and reject it at Lrun - 1.
+    p = 255
+    Lrun = forward_lrun(512, p)
+    ref255, mag255 = (t.view(8, 512, 768)[:, p] for t in (ref, mag))
+    for lr, wrong in ((Lrun, False), (Lrun - 1, True)):
+        y = run_biscan_ex_ok(lib, si, Lrun=lr)["y"]
+        st = Stats().add(y.t.view(8, 512, 768)[:, p], ref255, mag255, u_out, u_acc)
+        print(f"[bounds] self-check early stop: row {p} at Lrun = {lr} (valid rows [{512 - lr}, {lr})) -> max err/unit {st.ratio:.4g}")
+        assert rejects("scan_bf16", st) == wrong, lr
