@@ -75,10 +75,15 @@ int pcad_abi_version(void);
 /* Replaces: load_state_dict.  `name` is the checkpoint key (see plantcaduceus_b200/weights.py);
  * `data` may be a host or device pointer (unified addressing); src_dtype is a pcad_dtype.
  * The engine copies and re-lays-out; the caller keeps ownership. mamba_rev.{in,out}_proj alias
- * mamba_fwd's and are accepted and ignored. */
+ * mamba_fwd's and are accepted and ignored.
+ * A live handle may be reloaded: set_weight un-finalizes it and drops its CUDA graphs.  pcad_set_weight,
+ * pcad_finalize and pcad_set_tokenizer are load-time calls: each first synchronises the handle's device, so work
+ * already enqueued on any stream (forwards, graph replays) completes with the weights and tables it was enqueued with. */
 int pcad_set_weight(pcad_handle* h, const char* name, const void* data,
                     const int64_t* shape, int ndim, int src_dtype);
-/* Checks every weight is present, derives A = -exp(A_log) etc.  Must precede any forward. */
+/* Checks every weight is present, derives A = -exp(A_log) etc.  Must precede any forward.  Without
+ * lm_head.lm_head.weight the LM head is tied: every finalize derives it from the embedding as it then is (a reloaded
+ * embedding moves the head with it); once lm_head.lm_head.weight has been set on this handle, that is the head. */
 int pcad_finalize(pcad_handle* h);
 
 /* Tokeniser tables (replaces tokenizer.get_vocab() / mask_token_id, zero_shot_score.py:57,118):
@@ -155,6 +160,8 @@ int pcad_set_profiling(pcad_handle* h, int enabled);
 int pcad_get_profile(pcad_handle* h, float ms[PCAD_ST_COUNT], int64_t launches[PCAD_ST_COUNT]);
 /* Total kernels launched by this handle since creation. */
 int64_t pcad_launch_count(const pcad_handle* h);
+/* Score calls (pcad_score_windows_host / _dev) since creation that replayed a CUDA graph captured by an earlier call. */
+int64_t pcad_graph_replays(const pcad_handle* h);
 
 /* ---- single-operator entry points (device pointers; used by the parity tests and profiling) ----
  * All shapes are row-major, "token-major": activations are [rows, channels]. dtype is a pcad_dtype

@@ -90,7 +90,8 @@ struct pcad_handle {
   void* emb = nullptr;        // [V, d] act dtype
   float* head_w = nullptr;    // [V, d] fp32
   float* norm_f = nullptr;    // [d]
-  bool has_emb = false, has_head = false, has_norm_f = false;
+  bool has_emb = false, has_norm_f = false;
+  bool head_set = false;      // lm_head.lm_head.weight was set: otherwise every finalize derives the tied head from emb
   uint8_t* comp_dev = nullptr;   // [V]
   uint8_t* lut_dev = nullptr;    // [256]
   int* sel_dev = nullptr;        // [4] acgt ids
@@ -111,6 +112,7 @@ struct pcad_handle {
   cudaStream_t gstream = nullptr;       // capture / replay stream (the caller's may be the legacy default stream, which cannot capture)
   cudaEvent_t g_in = nullptr, g_out = nullptr;
   long long graph_max_tokens = 65536;   // strand-tokens (2 B L) up to which a forward is replayed from a graph
+  int64_t graph_replays = 0;            // calls served by a graph captured on an earlier call
   // profiling
   bool profiling = false;
   std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> prof_events;
@@ -940,6 +942,7 @@ int pcad_set_tokenizer(pcad_handle* h, const uint8_t lut[256], int mask_id, cons
   for (int i = 0; i < 256; ++i) if (lut[i] >= h->V) return fail(h, PCAD_ERR_INVALID, "lut[%d]=%d out of range", i, lut[i]);
   for (int k = 0; k < 4; ++k) if (acgt_ids[k] < 0 || acgt_ids[k] >= h->V) return fail(h, PCAD_ERR_INVALID, "acgt id out of range");
   CUDA_TRY(h, cudaSetDevice(h->device));
+  CUDA_TRY(h, cudaDeviceSynchronize());   // forwards and graph replays still queued on any stream read the old tables
   CUDA_TRY(h, cudaMemcpy(h->lut_dev, lut, 256, cudaMemcpyHostToDevice));
   int sel[4] = {acgt_ids[0], acgt_ids[1], acgt_ids[2], acgt_ids[3]};
   CUDA_TRY(h, cudaMemcpy(h->sel_dev, sel, sizeof(sel), cudaMemcpyHostToDevice));
@@ -953,6 +956,7 @@ int pcad_set_weight(pcad_handle* h, const char* name, const void* data, const in
   if (!h || !name || !data || !shape) return PCAD_ERR_INVALID;
   if (src_dtype != PCAD_BF16 && src_dtype != PCAD_F32 && src_dtype != PCAD_F16) return fail(h, PCAD_ERR_INVALID, "bad src_dtype for %s", name);
   CUDA_TRY(h, cudaSetDevice(h->device));
+  CUDA_TRY(h, cudaDeviceSynchronize());   // forwards and graph replays still queued on any stream read the old weights
   h->finalized = false;
   clear_graphs(h);
   const int d = h->d, E = h->E, N = h->N, R = h->R, V = h->V;
@@ -967,7 +971,7 @@ int pcad_set_weight(pcad_handle* h, const char* name, const void* data, const in
   if (s == "lm_head.lm_head.weight") {
     if (!shape_is(shape, ndim, {V, d})) return bad_shape();
     int rc = ingest(h, data, src_dtype, h->head_w, true, static_cast<long long>(V) * d);
-    h->has_head = rc == PCAD_OK;
+    h->head_set = rc == PCAD_OK;
     return rc;
   }
   if (s == "caduceus.backbone.norm_f.weight") {
@@ -1060,13 +1064,13 @@ int pcad_finalize(pcad_handle* h) {
   if (!h) return PCAD_ERR_INVALID;
   if (!h->has_emb) return fail(h, PCAD_ERR_MISSING, "missing weight: embedding");
   if (!h->has_norm_f) return fail(h, PCAD_ERR_MISSING, "missing weight: norm_f");
-  if (!h->has_head) {  // tied LM head (SURVEY.md Appendix A item 7): derive from the embedding
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  CUDA_TRY(h, cudaDeviceSynchronize());   // queued forwards read head_w and in_proj_s
+  if (!h->head_set) {  // tied LM head (SURVEY.md Appendix A item 7): derive from the (possibly reloaded) embedding
     const long long n = static_cast<long long>(h->V) * h->d;
-    CUDA_TRY(h, cudaSetDevice(h->device));
     if (h->f32) convert_kernel<float, float><<<static_cast<unsigned>((n + 255) / 256), 256>>>(static_cast<const float*>(h->emb), h->head_w, n);
     else convert_kernel<bf16, float><<<static_cast<unsigned>((n + 255) / 256), 256>>>(static_cast<const bf16*>(h->emb), h->head_w, n);
     CUDA_TRY(h, cudaDeviceSynchronize());
-    h->has_head = true;
   }
   static const char* names1[8] = {"conv1d.weight", "conv1d.bias", "x_proj.weight", "dt_proj.weight", "dt_proj.bias", "A_log", "D", nullptr};
   static const char* names2[8] = {"conv1d.weight", "conv1d.bias", nullptr, nullptr, "dt_bias", "A_log", "D", "norm.weight"};
@@ -1081,7 +1085,6 @@ int pcad_finalize(pcad_handle* h) {
         if (names[k] && !lw.dir[dir].has[k]) return fail(h, PCAD_ERR_MISSING, "missing weight: layers.%d mamba_%s.%s", li, dir ? "rev" : "fwd", names[k]);
   }
   if (h->fuse_norm) {
-    CUDA_TRY(h, cudaSetDevice(h->device));
     const long long rows = h->m2 ? h->DIP : 2LL * h->E, n = rows * h->d;
     for (auto& lw : h->layers)
       scale_columns_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(static_cast<const bf16*>(lw.in_proj), lw.norm_w,
@@ -1161,6 +1164,7 @@ int score_core_graphed(pcad_handle* h, int B, int L, int token_idx, cudaStream_t
       return score_core(h, B, L, token_idx, st);
     }
   }
+  const bool captured_before = !e->seen_only;
   if (e->seen_only) {
     const int64_t before = h->launch_count;
     cudaGraph_t graph = nullptr;
@@ -1187,6 +1191,7 @@ int score_core_graphed(pcad_handle* h, int B, int L, int token_idx, cudaStream_t
   CUDA_TRY(h, cudaEventRecord(h->g_out, h->gstream));
   CUDA_TRY(h, cudaStreamWaitEvent(st, h->g_out, 0));
   h->launch_count += e->launches;
+  if (captured_before) ++h->graph_replays;
   return PCAD_OK;
 }
 }  // namespace
@@ -1321,6 +1326,8 @@ int pcad_get_profile(pcad_handle* h, float ms[PCAD_ST_COUNT], int64_t launches[P
 }
 
 int64_t pcad_launch_count(const pcad_handle* h) { return h ? h->launch_count : 0; }
+
+int64_t pcad_graph_replays(const pcad_handle* h) { return h ? h->graph_replays : 0; }
 
 int pcad_op_sumsq_parts(int N) { return N > 0 ? gemm_sumsq_parts(N) : 0; }
 
