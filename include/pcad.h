@@ -118,6 +118,30 @@ int pcad_score_masked_at(pcad_handle* h, const uint8_t* ids_dev, int token_idx, 
 int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos,
                    void* hidden_dev, void* stream);
 
+/* Intermediate hidden states.  Replaces: model(input_ids, output_hidden_states=True).hidden_states[k], which has
+ * n_layer + 1 entries, each [B, L, 2*d_model] in the model dtype and in the layout of pcad_forward's hidden_dev (forward
+ * half, then the RC half with sequence and channels reversed back):
+ *   k = 0                the RCPS embedding;
+ *   k in [1, n_layer)    layer k-1's mixer output: out_proj's result before the residual add, the tensor layer k receives;
+ *   k = n_layer          the final normed state (pcad_forward's hidden_dev).
+ * tap_idx: n_taps host int32 indices, strictly increasing, in [0, n_layer]; tap_dev: host array of n_taps device pointers,
+ * tap i receives hidden_states[tap_idx[i]].  The ids are checked as pcad_forward checks them.  Taps change no other output
+ * bit: logits and every tap equal those of a call that requests any other set of taps, or none.  With logits_dev NULL the
+ * forward stops after the layer that produces the deepest requested entry (about k / n_layer of the full cost) and runs
+ * the final norm only if n_layer is requested.  Each tap is a caller buffer of B * L * 2 * d_model elements: with all
+ * 33 entries of PlantCaduceus_l32 (d_model 1024, bf16) at B = 256, L = 512 that is 33 x 0.54 GB = 17.7 GB.
+ * Returns PCAD_ERR_INVALID, before launching anything, for n_taps outside [1, n_layer + 1], an index outside
+ * [0, n_layer], indices not strictly increasing, or a null tap pointer.  Never uses a CUDA graph. */
+int pcad_forward_taps(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* logits_dev, int n_taps,
+                      const int32_t* tap_idx, void* const* tap_dev, void* stream);
+
+/* Replaces: hidden_states[k][:, tokenIdx, :] for the n_taps indices tap_idx (as pcad_forward_taps) without [B, L, 2*d_model]
+ * buffers: ids_dev uint8 [B, L], pos_dev int32 [B, n_pos]; hidden_dev receives [n_taps, B, n_pos, 2*d_model] in the model
+ * dtype, bit-identical to the matching slices of pcad_forward_taps.  Always stops at the deepest requested entry.  Same
+ * argument checks as pcad_forward_taps (hidden_dev is the tap pointer). */
+int pcad_hidden_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos,
+                          int n_taps, const int32_t* tap_idx, void* hidden_dev, void* stream);
+
 /* Token ids outside [0, vocab_size) (the reference's nn.Embedding would raise) are detected on the device by
  * pcad_forward / pcad_score_masked: the offending position is scored as id 0 and a flag is raised in mapped host
  * memory.  pcad_take_id_error returns PCAD_ERR_INVALID and clears the flag if any call since the last take saw such an
@@ -178,11 +202,17 @@ int pcad_op_linear(const void* A, const void* W, void* C, int64_t M, int N, int 
  *   pcad_op_linear_residual:  resid_out = A W^T + resid_in  (fp32 sum, stored bf16; resid_out may alias resid_in),
  *                             sumsq_out[row][p] = sum over column tile p of (fp32 sum)^2; float [M, pcad_op_sumsq_parts(N)],
  *                             every slot is written with a plain store (no atomics: results are deterministic)
+ *   pcad_op_linear_residual_tap: pcad_op_linear_residual, and also tap_out = bf16(A W^T) (row pitch ld_tap, 16-byte
+ *                             aligned, not aliasing the other operands), the sum before the residual add; tap_out equals
+ *                             pcad_op_linear's C and resid_out / sumsq_out equal pcad_op_linear_residual's, bit for bit
  *   pcad_op_linear_rowscale:  C = (A W^T) * rsqrt(sum_p sumsq_in[row][p] / K + eps)   -- RMSNorm of A's rows applied
  *                             after the GEMM; the norm weight must be pre-multiplied into W's columns by the caller. */
 int pcad_op_sumsq_parts(int N);
 int pcad_op_linear_residual(const void* A, const void* W, const void* resid_in, void* resid_out, float* sumsq_out,
                             int64_t M, int N, int K, int64_t lda, int64_t ldw, int64_t ld_res, int dtype, void* stream);
+int pcad_op_linear_residual_tap(const void* A, const void* W, const void* resid_in, void* resid_out, float* sumsq_out,
+                                void* tap_out, int64_t M, int N, int K, int64_t lda, int64_t ldw, int64_t ld_res,
+                                int64_t ld_tap, int dtype, void* stream);
 int pcad_op_linear_rowscale(const void* A, const void* W, const float* sumsq_in, int sumsq_parts, float eps, void* C,
                             int64_t M, int N, int K, int64_t lda, int64_t ldw, int64_t ldc, int dtype, void* stream);
 

@@ -20,10 +20,11 @@ ABI_VERSION = 3
 
 EXPORTS = (
     "pcad_abi_version", "pcad_create", "pcad_destroy", "pcad_last_error", "pcad_set_weight", "pcad_finalize",
-    "pcad_set_tokenizer", "pcad_take_id_error", "pcad_hidden_at", "pcad_forward", "pcad_score_masked", "pcad_score_masked_at", "pcad_score_windows_host", "pcad_score_windows_dev", "pcad_extract_windows", "pcad_tokenize",
+    "pcad_set_tokenizer", "pcad_take_id_error", "pcad_hidden_at", "pcad_forward",
+    "pcad_forward_taps", "pcad_hidden_at_layers", "pcad_score_masked", "pcad_score_masked_at", "pcad_score_windows_host", "pcad_score_windows_dev", "pcad_extract_windows", "pcad_tokenize",
     "pcad_workspace_bytes", "pcad_set_profiling", "pcad_get_profile", "pcad_launch_count",
     "pcad_graph_replays",
-    "pcad_op_linear", "pcad_op_linear_residual", "pcad_op_linear_rowscale", "pcad_op_sumsq_parts",
+    "pcad_op_linear", "pcad_op_linear_residual", "pcad_op_linear_residual_tap", "pcad_op_linear_rowscale", "pcad_op_sumsq_parts",
     "pcad_op_add_rmsnorm", "pcad_op_conv_silu", "pcad_op_biscan", "pcad_op_biscan_segmented", "pcad_op_biscan_ex",
     "pcad_op_biscan_dt",
     "pcad_op_ssd_scan", "pcad_op_gated_norm_sum",
@@ -70,6 +71,8 @@ def load() -> C.CDLL:
     lib.pcad_take_id_error.argtypes = [vp, vp, i32]
     lib.pcad_hidden_at.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
     lib.pcad_forward.argtypes = [vp, vp, i32, i32, vp, vp, vp]
+    lib.pcad_forward_taps.argtypes = [vp, vp, i32, i32, vp, i32, C.POINTER(C.c_int32), C.POINTER(vp), vp]
+    lib.pcad_hidden_at_layers.argtypes = [vp, vp, vp, i32, i32, i32, i32, C.POINTER(C.c_int32), vp, vp]
     lib.pcad_score_masked.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
     lib.pcad_score_masked_at.argtypes = [vp, vp, i32, i32, i32, vp, vp]
     lib.pcad_score_windows_host.argtypes = [vp, vp, i32, i32, i32, vp, vp]
@@ -85,6 +88,7 @@ def load() -> C.CDLL:
     lib.pcad_graph_replays.restype = i64
     lib.pcad_op_linear.argtypes = [vp, vp, vp, i64, i32, i32, i64, i64, i64, i32, vp]
     lib.pcad_op_linear_residual.argtypes = [vp, vp, vp, vp, vp, i64, i32, i32, i64, i64, i64, i32, vp]
+    lib.pcad_op_linear_residual_tap.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, i32, i64, i64, i64, i64, i32, vp]
     lib.pcad_op_linear_rowscale.argtypes = [vp, vp, vp, i32, C.c_float, vp, i64, i32, i32, i64, i64, i64, i32, vp]
     lib.pcad_op_sumsq_parts.argtypes = [i32]
     lib.pcad_op_add_rmsnorm.argtypes = [vp, vp, vp, vp, vp, i64, i32, C.c_float, i32, i32, vp]

@@ -52,7 +52,14 @@ struct GemmCfg {
 //                            forward is deterministic and the two strands stay bit-identical;
 //   in_proj,  kEpiRowScale:  C = acc * rsqrt(sum_parts sumsq[row][.] / K + eps), with the norm weight pre-multiplied
 //                            into the columns of W at load time: (r * rstd * w) W^T == rstd * (r (W diag(w))^T).
-enum { kEpiPlain = 0, kEpiResidual = 2, kEpiRowScale = 3 };
+//   out_proj, kEpiResidualTap: kEpiResidual, and also tap[row] = bf16(acc), the block's mixer output before the residual
+//                            add (the reference's intermediate hidden_states entry).  The same accumulator is rounded once
+//                            for the tap and once, after the add, for the residual stream, so the stream and everything
+//                            downstream are bit-identical to kEpiResidual's, and the tap to kEpiPlain's.  Each lane stores
+//                            its row's 16-byte pieces straight to global memory, next to the residual loads it already
+//                            makes: a TMA store would need a second tensor map in the kernel's arguments (changing every
+//                            other instantiation) and a second staging slab in shared memory.
+enum { kEpiPlain = 0, kEpiResidual = 2, kEpiRowScale = 3, kEpiResidualTap = 4 };
 
 struct EpiParams {
   const bf16* resid = nullptr;        // kEpiResidual: [M, N] with row pitch ld_res (may alias C)
@@ -62,6 +69,8 @@ struct EpiParams {
   int sumsq_parts = 1;
   float inv_k = 0.f;                  // kEpiRowScale: 1 / (row length the sum of squares was taken over)
   float eps = 0.f;
+  bf16* tap = nullptr;                // kEpiResidualTap: [M, N] with row pitch ld_tap, bf16(acc) before the residual add
+  long long ld_tap = 0;
 };
 
 template <int BN, int EPI, int EW, int CG>
@@ -70,6 +79,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                          const __grid_constant__ CUtensorMap tmap_c, long long M, int N, int K, const EpiParams ep) {
   using Cfg = GemmCfg<BN, EW, CG>;
   constexpr int STAGES = Cfg::kStages;
+  constexpr bool kResid = EPI == kEpiResidual || EPI == kEpiResidualTap;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* ring = smem;
@@ -210,7 +220,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         __syncwarp();
         uint32_t r0[32], r1[32];
         uint4 res[8];
-        if constexpr (EPI == kEpiResidual) {   // this row's 64 residual values: issued before the TMEM load returns
+        if constexpr (kResid) {   // this row's 64 residual values: issued before the TMEM load returns
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             const int col = n0 + c0 + j * 8;
@@ -221,12 +231,22 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         tmem_ld_32x32b_x32(t_row + c0, r0);
         if (c0 + 32 < BN) tmem_ld_32x32b_x32(t_row + c0 + 32, r1);
         tmem_ld_wait();
-        if constexpr (EPI == kEpiResidual) {
+        if constexpr (kResid) {
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             uint32_t* r = (j < 4) ? (r0 + j * 8) : (r1 + (j - 4) * 8);
             const uint32_t w[4] = {res[j].x, res[j].y, res[j].z, res[j].w};
             const bool col_ok = n0 + c0 + j * 8 + 8 <= N;
+            if constexpr (EPI == kEpiResidualTap) {
+              if (row_ok && col_ok) {
+                uint4 t;
+                t.x = pack_bf16x2(__uint_as_float(r[0]), __uint_as_float(r[1]));
+                t.y = pack_bf16x2(__uint_as_float(r[2]), __uint_as_float(r[3]));
+                t.z = pack_bf16x2(__uint_as_float(r[4]), __uint_as_float(r[5]));
+                t.w = pack_bf16x2(__uint_as_float(r[6]), __uint_as_float(r[7]));
+                *reinterpret_cast<uint4*>(ep.tap + grow * ep.ld_tap + n0 + c0 + j * 8) = t;
+              }
+            }
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
               const float v0 = __uint_as_float(r[2 * k]) + __uint_as_float(w[k] << 16);
@@ -266,8 +286,8 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
       }
       tc_fence_before();
       if constexpr (CG == 2) mbar_arrive_leader(&tmem_empty[acc]); else mbar_arrive(&tmem_empty[acc]);
-      if constexpr (EPI == kEpiResidual) {
-        static_assert(EPI != kEpiResidual || EW == 4, "one sum-of-squares slot per column tile assumes one warp per lane quarter");
+      if constexpr (kResid) {
+        static_assert(!kResid || EW == 4, "one sum-of-squares slot per column tile assumes one warp per lane quarter");
         if (row_ok) ep.sumsq_out[grow * ep.sumsq_parts + (n0 / BN)] = row_ss;
       }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
@@ -363,12 +383,17 @@ inline cudaError_t gemm_bf16_tcgen05(const bf16* A, const bf16* W, bf16* C, long
     *why = "gemm: pointers must be 16-byte aligned and row pitches multiples of 8 elements";
     return cudaErrorInvalidValue;
   }
-  if (epi == kEpiResidual && (!ep.resid || !ep.sumsq_out || (N % 8) || (ep.ld_res % 8) ||
-                              (reinterpret_cast<uintptr_t>(ep.resid) & 15))) {
+  const bool resid_epi = epi == kEpiResidual || epi == kEpiResidualTap;
+  if (resid_epi && (!ep.resid || !ep.sumsq_out || (N % 8) || (ep.ld_res % 8) ||
+                    (reinterpret_cast<uintptr_t>(ep.resid) & 15))) {
     *why = "gemm: the residual epilogue needs resid (16-byte aligned, pitch % 8 == 0), sumsq_out and N % 8 == 0";
     return cudaErrorInvalidValue;
   }
-  if (epi == kEpiResidual && ep.sumsq_parts != gemm_sumsq_parts(N)) {
+  if (epi == kEpiResidualTap && (!ep.tap || (ep.ld_tap % 8) || ep.ld_tap < N || (reinterpret_cast<uintptr_t>(ep.tap) & 15))) {
+    *why = "gemm: the residual tap epilogue needs tap (16-byte aligned, pitch % 8 == 0 and >= N)";
+    return cudaErrorInvalidValue;
+  }
+  if (resid_epi && ep.sumsq_parts != gemm_sumsq_parts(N)) {
     *why = "gemm: sumsq_parts must equal gemm_sumsq_parts(N)";
     return cudaErrorInvalidValue;
   }
@@ -387,6 +412,7 @@ inline cudaError_t gemm_bf16_tcgen05(const bf16* A, const bf16* W, bf16* C, long
   if (pair) {
     switch (epi) {
       case kEpiResidual: return launch_gemm_bn<256, kEpiResidual, 4, 2>(ta, tb, tc, M, N, K, ep, num_sms, stream);
+      case kEpiResidualTap: return launch_gemm_bn<256, kEpiResidualTap, 4, 2>(ta, tb, tc, M, N, K, ep, num_sms, stream);
       case kEpiRowScale: return launch_gemm_bn<256, kEpiRowScale, 4, 2>(ta, tb, tc, M, N, K, ep, num_sms, stream);
       default: return launch_gemm_bn<256, kEpiPlain, 4, 2>(ta, tb, tc, M, N, K, ep, num_sms, stream);
     }
@@ -394,6 +420,7 @@ inline cudaError_t gemm_bf16_tcgen05(const bf16* A, const bf16* W, bf16* C, long
 #define PCAD_GEMM_EPI(BNV)                                                                                  \
   switch (epi) {                                                                                            \
     case kEpiResidual: return launch_gemm_bn<BNV, kEpiResidual>(ta, tb, tc, M, N, K, ep, num_sms, stream);  \
+    case kEpiResidualTap: return launch_gemm_bn<BNV, kEpiResidualTap>(ta, tb, tc, M, N, K, ep, num_sms, stream); \
     case kEpiRowScale: return launch_gemm_bn<BNV, kEpiRowScale>(ta, tb, tc, M, N, K, ep, num_sms, stream);  \
     default: return launch_gemm_bn<BNV, kEpiPlain>(ta, tb, tc, M, N, K, ep, num_sms, stream);               \
   }

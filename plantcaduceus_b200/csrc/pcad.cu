@@ -605,13 +605,55 @@ __global__ void gather_rows_kernel(const uint4* __restrict__ src, uint4* __restr
   dst[gid] = src[(static_cast<long long>(s) * L + row) * vec_per_row + v];
 }
 
+// ---- hidden-state taps ---------------------------------------------------------------------------------
+// Which entries of the reference's hidden_states tuple a forward emits, and where: idx[i] (strictly increasing, in
+// [0, n_layer]) goes to dst[i], [B, L, 2d] in the model dtype; or, with pos, [B, n_pos, 2d] at the positions pos[b, :].
+struct Taps {
+  int n = 0;
+  const int32_t* idx = nullptr;
+  void* const* dst = nullptr;
+  const int32_t* pos = nullptr;   // device, [B, n_pos]; nullptr: every position
+  int n_pos = 0;
+  int deepest() const { return n > 0 ? idx[n - 1] : -1; }
+  int find(int k) const {   // i with idx[i] == k, or -1
+    for (int i = 0; i < n; ++i)
+      if (idx[i] == k) return i;
+    return -1;
+  }
+};
+
+// Writes hidden_states[k] from the strand-major [2BL, d] rows `src` into dst[i] if k is tap i (hidden_tap_kernel /
+// hidden_tap_pos_kernel: the RC half reversed in time and channels).
+int emit_tap(pcad_handle* h, const Taps* taps, int k, const void* src, int B, int L, cudaStream_t st) {
+  const int i = taps ? taps->find(k) : -1;
+  if (i < 0) return PCAD_OK;
+  StageTimer tm(h, st, PCAD_ST_MISC);
+  const int d = h->d;
+  if (taps->pos) {
+    const long long total = static_cast<long long>(B) * taps->n_pos * (2 * d / 8);
+    const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
+    if (h->f32) hidden_tap_pos_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(src), taps->pos, taps->n_pos, static_cast<float*>(taps->dst[i]), B, L, d);
+    else hidden_tap_pos_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(src), taps->pos, taps->n_pos, static_cast<bf16*>(taps->dst[i]), B, L, d);
+  } else {
+    const long long total = static_cast<long long>(B) * L * (2 * d / 8);
+    const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
+    if (h->f32) hidden_tap_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(src), static_cast<float*>(taps->dst[i]), B, L, d);
+    else hidden_tap_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(src), static_cast<bf16*>(taps->dst[i]), B, L, d);
+  }
+  CUDA_TRY(h, cudaGetLastError());
+  return PCAD_OK;
+}
+
 // ---- the forward pass over the strand-major layout --------------------------------------------------
 // ids (u8 [B, L]) are already in ws.ids.  Leaves the final normed hidden state in ws.normed.
 // prune_idx >= 0 (score-only calls with one scored position per window): the LAST layer is computed only as far as the head
 // needs it -- the scan stops once both directions have reached the scored position (about half the steps at the window centre),
 // out_proj / residual / final norm run on the 2B rows the head reads, and ws.normed comes back COMPACT as [2B, d] (the head is then
 // called with L = 1, position 0).  Bit-identical to the full computation at those rows.
-int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = -1) {
+// taps (never with prune_idx): the hidden_states entries to emit as each comes into existence -- 0 the embedding, k in
+// [1, n_layer) layer k-1's out_proj output before the residual add, n_layer the final norm.  With full = false the forward
+// stops after the layer that produces the deepest requested entry, and runs the final norm only if n_layer is requested.
+int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = -1, const Taps* taps = nullptr, bool full = true) {
   Workspace& ws = h->ws;
   const long long T = 2LL * B * L;
   const int S = 2 * B;
@@ -642,9 +684,12 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
     if (fused) row_sumsq_kernel<<<static_cast<unsigned>((T + 7) / 8), 256, 0, st>>>(static_cast<const bf16*>(ws.resid), ws.sumsq[cur], T, d, parts);
     CUDA_TRY(h, cudaGetLastError());
   }
-  for (int li = 0; li < h->cfg.n_layer; ++li) {
+  int rc = emit_tap(h, taps, 0, x, B, L, st);
+  if (rc) return rc;
+  const int n_layer = h->cfg.n_layer;
+  const int n_run = full || !taps ? n_layer : (taps->deepest() < n_layer ? taps->deepest() : n_layer);
+  for (int li = 0; li < n_run; ++li) {
     LayerWeights& lw = h->layers[li];
-    int rc;
     if (!fused) {
       StageTimer tm(h, st, PCAD_ST_NORM);
       rc = op_add_rmsnorm(h, ws.hid, li == 0 ? nullptr : ws.resid, lw.norm_w, ws.normed, ws.resid, T, d, h->cfg.norm_eps, f32, res_f32, st);
@@ -688,26 +733,40 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
       res = rc_in;
       x = rc_in + align_up(static_cast<size_t>(S) * d * 4, 1024);                       // [S, d]   new residual / out_proj output
     }
+    // hidden_states[li + 1] is this layer's out_proj output (the last layer's is not an entry: index n_layer is the final norm)
+    const bool tap_here = taps && li + 1 < n_layer && taps->find(li + 1) >= 0;
     {
       StageTimer tm(h, st, PCAD_ST_OUT_PROJ);
       if (fused) {
+        // the fused path never stores the pre-residual output, except as the tap: into ws.hid, which it does not otherwise use
         EpiParams ep;
         ep.resid = static_cast<const bf16*>(res);
         ep.ld_res = d;
         ep.sumsq_out = ws.sumsq[cur ^ 1];
         ep.sumsq_parts = parts;
-        rc = op_linear(h, y, lw.out_proj, x, rows, d, E, E, E, d, false, h->num_sms, st, kEpiResidual, ep);
+        ep.tap = static_cast<bf16*>(ws.hid);
+        ep.ld_tap = d;
+        rc = op_linear(h, y, lw.out_proj, x, rows, d, E, E, E, d, false, h->num_sms, st, tap_here ? kEpiResidualTap : kEpiResidual, ep);
         cur ^= 1;
       } else {
         rc = op_linear(h, y, lw.out_proj, x, rows, d, E, E, E, d, f32, h->num_sms, st);
       }
       if (rc) return rc;
     }
+    if (tap_here) {
+      rc = emit_tap(h, taps, li + 1, ws.hid, B, L, st);
+      if (rc) return rc;
+    }
   }
-  // the fused path has already added the residual in out_proj's epilogue; without a layer there is no residual yet
-  StageTimer tm(h, st, PCAD_ST_NORM);
-  return op_add_rmsnorm(h, x, fused || h->cfg.n_layer == 0 ? nullptr : res, h->norm_f, ws.normed, nullptr, rows, d, h->cfg.norm_eps,
+  if (n_run < n_layer) return PCAD_OK;   // stopped early: the final norm is not requested
+  {
+    // the fused path has already added the residual in out_proj's epilogue; without a layer there is no residual yet
+    StageTimer tm(h, st, PCAD_ST_NORM);
+    rc = op_add_rmsnorm(h, x, fused || n_layer == 0 ? nullptr : res, h->norm_f, ws.normed, nullptr, rows, d, h->cfg.norm_eps,
                         f32, res_f32, st);
+    if (rc) return rc;
+  }
+  return emit_tap(h, taps, n_layer, ws.normed, B, L, st);
 }
 
 int run_head(pcad_handle* h, int B, int L, const int* pos_dev, int n_pos, float* out, cudaStream_t st) {
@@ -755,6 +814,27 @@ int stage_ids(pcad_handle* h, const uint8_t* ids_dev, int B, int L, int token_id
     fill_int_kernel<<<(B + 255) / 256, 256, 0, st>>>(ws.pos0, B, 0);
   }
   CUDA_TRY(h, cudaGetLastError());
+  return PCAD_OK;
+}
+
+// ids (int64 [B, L], device) -> ws.ids, checked as stage_ids does.
+int stage_ids64(pcad_handle* h, const int64_t* ids_dev, int B, int L, cudaStream_t st) {
+  StageTimer tm(h, st, PCAD_ST_MISC);
+  const long long n = static_cast<long long>(B) * L;
+  ids64_to_u8_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<const long long*>(ids_dev), h->ws.ids, n, h->V, h->bad_flag);
+  CUDA_TRY(h, cudaGetLastError());
+  return PCAD_OK;
+}
+
+// The tap list of pcad_forward_taps / pcad_hidden_at_layers, checked before anything is launched.
+int check_taps(pcad_handle* h, int n_taps, const int32_t* tap_idx) {
+  const int n_layer = h->cfg.n_layer;
+  if (n_taps < 1 || n_taps > n_layer + 1) return fail(h, PCAD_ERR_INVALID, "n_taps = %d outside [1, n_layer + 1 = %d]", n_taps, n_layer + 1);
+  if (!tap_idx) return fail(h, PCAD_ERR_INVALID, "tap_idx is null");
+  for (int i = 0; i < n_taps; ++i) {
+    if (tap_idx[i] < 0 || tap_idx[i] > n_layer) return fail(h, PCAD_ERR_INVALID, "tap_idx[%d] = %d outside [0, n_layer = %d]", i, tap_idx[i], n_layer);
+    if (i > 0 && tap_idx[i] <= tap_idx[i - 1]) return fail(h, PCAD_ERR_INVALID, "tap_idx is not strictly increasing at %d", i);
+  }
   return PCAD_OK;
 }
 
@@ -1213,12 +1293,8 @@ int pcad_forward(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* lo
   int rc = begin_call(h, B, L, 1, ids_dev, "ids_dev is null");
   if (rc) return rc == kNoWork ? PCAD_OK : rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  {
-    StageTimer tm(h, st, PCAD_ST_MISC);
-    const long long n = static_cast<long long>(B) * L;
-    ids64_to_u8_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<const long long*>(ids_dev), h->ws.ids, n, h->V, h->bad_flag);
-    CUDA_TRY(h, cudaGetLastError());
-  }
+  rc = stage_ids64(h, ids_dev, B, L, st);
+  if (rc) return rc;
   rc = run_backbone(h, B, L, st);
   if (rc) return rc;
   if (logits_dev) {
@@ -1271,6 +1347,52 @@ int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_de
   else hidden_tap_pos_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(h->ws.normed), pos_dev, n_pos, static_cast<bf16*>(hidden_dev), B, L, h->d);
   CUDA_TRY(h, cudaGetLastError());
   return PCAD_OK;
+}
+
+int pcad_forward_taps(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* logits_dev, int n_taps, const int32_t* tap_idx,
+                      void* const* tap_dev, void* stream) {
+  if (!h) return PCAD_ERR_INVALID;
+  int rc = check_taps(h, n_taps, tap_idx);
+  if (rc) return rc;
+  if (!tap_dev) return fail(h, PCAD_ERR_INVALID, "tap_dev is null");
+  for (int i = 0; i < n_taps; ++i)
+    if (!tap_dev[i]) return fail(h, PCAD_ERR_INVALID, "tap_dev[%d] is null", i);
+  rc = begin_call(h, B, L, 1, ids_dev, "ids_dev is null");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = stage_ids64(h, ids_dev, B, L, st);
+  if (rc) return rc;
+  Taps taps;
+  taps.n = n_taps;
+  taps.idx = tap_idx;
+  taps.dst = tap_dev;
+  rc = run_backbone(h, B, L, st, -1, &taps, logits_dev != nullptr);
+  if (rc || !logits_dev) return rc;
+  return run_head(h, B, L, nullptr, 0, logits_dev, st);
+}
+
+int pcad_hidden_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos, int n_taps,
+                          const int32_t* tap_idx, void* hidden_dev, void* stream) {
+  if (!h) return PCAD_ERR_INVALID;
+  int rc = check_taps(h, n_taps, tap_idx);
+  if (rc) return rc;
+  if (!hidden_dev) return fail(h, PCAD_ERR_INVALID, "hidden_dev is null");
+  rc = begin_call(h, B, L, n_pos, ids_dev && pos_dev && n_pos >= 0, "null or negative argument");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = stage_ids(h, ids_dev, B, L, -1, st);
+  if (rc) return rc;
+  // tap i occupies [B, n_pos, 2d] of hidden_dev, after the i taps before it
+  const size_t tap_bytes = static_cast<size_t>(B) * n_pos * 2 * h->d * h->act_size;
+  std::vector<void*> dst(n_taps);
+  for (int i = 0; i < n_taps; ++i) dst[i] = static_cast<uint8_t*>(hidden_dev) + i * tap_bytes;
+  Taps taps;
+  taps.n = n_taps;
+  taps.idx = tap_idx;
+  taps.dst = dst.data();
+  taps.pos = pos_dev;
+  taps.n_pos = n_pos;
+  return run_backbone(h, B, L, st, -1, &taps, false);
 }
 
 int pcad_score_windows_host(pcad_handle* h, const uint8_t* ascii_host, int B, int L, int token_idx, float* logits4_host, void* stream) {
@@ -1361,6 +1483,19 @@ int pcad_op_linear_residual(const void* A, const void* W, const void* resid_in, 
   ep.sumsq_out = sumsq_out;
   ep.sumsq_parts = gemm_sumsq_parts(N);
   return op_fail_to_global(op_linear(op_scratch(), A, W, resid_out, M, N, K, lda, ldw, ld_res, false, op_num_sms(), static_cast<cudaStream_t>(stream), kEpiResidual, ep));
+}
+
+int pcad_op_linear_residual_tap(const void* A, const void* W, const void* resid_in, void* resid_out, float* sumsq_out, void* tap_out,
+                                int64_t M, int N, int K, int64_t lda, int64_t ldw, int64_t ld_res, int64_t ld_tap, int dtype, void* stream) {
+  if (dtype != PCAD_BF16 || !resid_in || !sumsq_out || !tap_out) return PCAD_ERR_INVALID;
+  EpiParams ep;
+  ep.resid = static_cast<const bf16*>(resid_in);
+  ep.ld_res = ld_res;
+  ep.sumsq_out = sumsq_out;
+  ep.sumsq_parts = gemm_sumsq_parts(N);
+  ep.tap = static_cast<bf16*>(tap_out);
+  ep.ld_tap = ld_tap;
+  return op_fail_to_global(op_linear(op_scratch(), A, W, resid_out, M, N, K, lda, ldw, ld_res, false, op_num_sms(), static_cast<cudaStream_t>(stream), kEpiResidualTap, ep));
 }
 
 int pcad_op_linear_rowscale(const void* A, const void* W, const float* sumsq_in, int sumsq_parts, float eps, void* C, int64_t M, int N, int K,

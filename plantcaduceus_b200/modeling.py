@@ -10,9 +10,10 @@ from __future__ import annotations
 
 import ctypes as C
 import json
+import numbers
 import os
 from dataclasses import dataclass
-from typing import Dict, Optional, Tuple, Union
+from typing import Dict, Iterable, List, Optional, Tuple, Union
 
 import numpy as np
 import torch
@@ -31,6 +32,36 @@ class MaskedLMOutput:
 
 
 _TORCH_TO_PCAD = {torch.float32: _lib.PCAD_F32, torch.bfloat16: _lib.PCAD_BF16, torch.float16: _lib.PCAD_F16}
+
+
+def hidden_layer_indices(layers: Union[str, Iterable[int]], n_layer: int) -> List[int]:
+    """Indices into the reference's ``hidden_states`` tuple (``n_layer + 1`` entries: 0 the embedding, k in [1, n_layer) layer
+    k-1's mixer output, n_layer the final normed state) in the caller's order, negative ones counted from the end as Python
+    does.  ``"all"`` is every index.  Raises ValueError for anything else than "all" or a non-empty iterable of ints, for an
+    index outside [-(n_layer + 1), n_layer], and for an index requested twice."""
+    n = n_layer + 1
+    if isinstance(layers, str):
+        if layers != "all":
+            raise ValueError(f"hidden layers must be 'all' or an iterable of ints, not {layers!r}")
+        return list(range(n))
+    try:
+        items = list(layers)
+    except TypeError:
+        raise ValueError(f"hidden layers must be 'all' or an iterable of ints, not {layers!r}") from None
+    if not items:
+        raise ValueError("no hidden layer requested")
+    out = []
+    for k in items:
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, numbers.Integral):
+            raise ValueError(f"hidden layer index {k!r} is not an int")
+        k = int(k)
+        if not -n <= k < n:
+            raise ValueError(f"hidden layer index {k} out of range for {n} hidden states (n_layer = {n_layer})")
+        k %= n
+        if k in out:
+            raise ValueError(f"hidden layer index {k} requested twice (after counting negative indices from the end)")
+        out.append(k)
+    return out
 
 
 class CaduceusForMaskedLM:
@@ -200,14 +231,20 @@ class CaduceusForMaskedLM:
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def __call__(self, input_ids: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
-                 return_dict: bool = True, **unused) -> MaskedLMOutput:
-        return self.forward(input_ids=input_ids, output_hidden_states=output_hidden_states)
+                 return_dict: bool = True, hidden_layers: Union[None, str, Iterable[int]] = None, **unused) -> MaskedLMOutput:
+        return self.forward(input_ids=input_ids, output_hidden_states=output_hidden_states, hidden_layers=hidden_layers)
 
     def forward(self, input_ids: torch.Tensor, output_hidden_states: bool = False,
-                compute_logits: bool = True) -> MaskedLMOutput:
+                compute_logits: bool = True, hidden_layers: Union[None, str, Iterable[int]] = None) -> MaskedLMOutput:
+        """``hidden_layers`` ("all", or indices into the reference's hidden_states, negative ones from the end) implies
+        ``output_hidden_states`` and returns the reference's full tuple of ``n_layer + 1`` entries, [B, L, 2*d_model] each,
+        the requested ones filled and the others None.  With ``compute_logits=False`` the forward then stops after the layer
+        that produces the deepest requested entry.  Without it, hidden_states holds the final normed state only."""
         self._require_handle()
         if input_ids is None or input_ids.dim() != 2:
             raise ValueError("input_ids must be a [batch, length] integer tensor")
+        if hidden_layers is not None:
+            return self._forward_taps(input_ids, hidden_layer_indices(hidden_layers, self.config.n_layer), compute_logits)
         ids = input_ids.to(device=self.device, dtype=torch.int64).contiguous()
         B, L = ids.shape
         with torch.cuda.device(self.device):
@@ -224,6 +261,27 @@ class CaduceusForMaskedLM:
         # hidden_states: only the final (normed) state is materialised; hidden_states[-1] is what the
         # reference's callers read (train_XGBoost.py:105, notebooks/examples.ipynb:183).
         return MaskedLMOutput(logits=logits, hidden_states=(hidden,) if hidden is not None else None)
+
+    def _forward_taps(self, input_ids: torch.Tensor, layers: List[int], compute_logits: bool) -> MaskedLMOutput:
+        ids = input_ids.to(device=self.device, dtype=torch.int64).contiguous()
+        B, L = ids.shape
+        want = sorted(layers)
+        with torch.cuda.device(self.device):
+            logits = torch.empty((B, L, self.config.vocab_size), dtype=torch.float32, device=self.device) \
+                if compute_logits else None
+            taps = [torch.empty((B, L, 2 * self.config.d_model), dtype=self.dtype, device=self.device) for _ in want]
+            if B > 0 and L > 0:
+                idx = (C.c_int32 * len(want))(*want)
+                ptrs = (C.c_void_p * len(want))(*[t.data_ptr() for t in taps])
+                _lib.check(self._lib.pcad_forward_taps(
+                    self._handle, C.c_void_p(ids.data_ptr()), B, L,
+                    C.c_void_p(logits.data_ptr()) if logits is not None else None, len(want), idx, ptrs,
+                    self._stream()), self._handle)
+                self._raise_on_bad_ids(True)
+        hidden: List[Optional[torch.Tensor]] = [None] * (self.config.n_layer + 1)
+        for k, t in zip(want, taps):
+            hidden[k] = t
+        return MaskedLMOutput(logits=logits, hidden_states=tuple(hidden))
 
     def _raise_on_bad_ids(self, sync: bool):
         """Token ids outside [0, vocab_size) raise IndexError, as the reference's nn.Embedding lookup would
@@ -262,10 +320,15 @@ class CaduceusForMaskedLM:
                 self._raise_on_bad_ids(check_ids)
         return out
 
-    def hidden_at(self, ids_u8: torch.Tensor, positions: torch.Tensor) -> torch.Tensor:
+    def hidden_at(self, ids_u8: torch.Tensor, positions: torch.Tensor,
+                  layers: Union[None, str, Iterable[int]] = None) -> torch.Tensor:
         """``hidden_states[-1][b, positions[b, i], :]`` for uint8 ids [B, L]: [B, n_pos, 2*d_model] in the model dtype,
-        without materialising the full hidden state (reference extract_embeddings, train_XGBoost.py:104-105)."""
+        without materialising the full hidden state (reference extract_embeddings, train_XGBoost.py:104-105).  With
+        ``layers`` ("all", or indices into hidden_states as ``forward``'s ``hidden_layers``): [len(layers), B, n_pos,
+        2*d_model], entry i from hidden_states[layers[i]]; the forward stops after the deepest requested layer."""
         self._require_handle()
+        if layers is not None:
+            return self._hidden_at_layers(ids_u8, positions, hidden_layer_indices(layers, self.config.n_layer))
         ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
         pos = positions.to(device=self.device, dtype=torch.int32).contiguous()
         B, L = ids.shape
@@ -278,6 +341,26 @@ class CaduceusForMaskedLM:
                 _lib.check(self._lib.pcad_hidden_at(self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(pos.data_ptr()),
                                                     B, L, n_pos, C.c_void_p(out.data_ptr()), self._stream()), self._handle)
                 self._raise_on_bad_ids(True)
+        return out
+
+    def _hidden_at_layers(self, ids_u8: torch.Tensor, positions: torch.Tensor, layers: List[int]) -> torch.Tensor:
+        ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
+        pos = positions.to(device=self.device, dtype=torch.int32).contiguous()
+        B, L = ids.shape
+        if pos.dim() == 1:
+            pos = pos[:, None]
+        n_pos = pos.shape[1]
+        want = sorted(layers)
+        with torch.cuda.device(self.device):
+            out = torch.empty((len(want), B, n_pos, 2 * self.config.d_model), dtype=self.dtype, device=self.device)
+            if B > 0 and L > 0 and n_pos > 0:
+                idx = (C.c_int32 * len(want))(*want)
+                _lib.check(self._lib.pcad_hidden_at_layers(self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(pos.data_ptr()),
+                                                           B, L, n_pos, len(want), idx, C.c_void_p(out.data_ptr()),
+                                                           self._stream()), self._handle)
+                self._raise_on_bad_ids(True)
+            if want != layers:   # the engine takes the indices in increasing order; return them in the caller's
+                out = out[torch.tensor([want.index(k) for k in layers], device=self.device)]
         return out
 
     def score_windows_host(self, ascii_windows: Union[np.ndarray, torch.Tensor], token_idx: int,
