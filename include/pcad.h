@@ -142,6 +142,31 @@ int pcad_forward_taps(pcad_handle* h, const int64_t* ids_dev, int B, int L, floa
 int pcad_hidden_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos,
                           int n_taps, const int32_t* tap_idx, void* hidden_dev, void* stream);
 
+/* Mean-pooled hidden states: one vector per window and per entry, the input of frozen-embedding classifiers and layer-wise
+ * probes.  For uint8 ids_dev [B, L], the n_taps indices tap_idx (as pcad_forward_taps) and per-window ranges [s_b, e_b):
+ *   out_dev[i, b, :] = mean over t in [s_b, e_b) of hidden_states[tap_idx[i]][b, t, :]        float32 [n_taps, B, 2*d_model]
+ * in the layout of hidden_states (forward half, then the RC half with its channels in the reference's order, so the
+ * caller's strand average applies as is).  ranges_dev: int32 [B, 2] on the device, (s_b, e_b) per window; NULL means
+ * [0, L) for every window.  A window whose range is invalid (s < 0, e > L or s >= e) gets a NaN row; the other rows are
+ * unaffected, and nothing waits on the host.  The states inside a range still see every position of the window, padding
+ * included, through the bidirectional scans, as they do in the reference: a range selects what is averaged, not what the
+ * model reads.
+ * Summation order, fixed: entries are read in the model dtype and summed in fp32, positions in reference order
+ * t = s, s+1, ...; sequentially within chunks of PCAD_HIDDEN_MEAN_CHUNK consecutive positions counted from s; the chunk
+ * partials then sequentially in chunk order; the total divided by (float)(e - s) with a correctly rounded division.  So a
+ * window's result depends neither on B, nor on the other windows, nor on which other entries are requested; it is
+ * bit-identical run to run, and no atomics are used.  A one-position range (e = s + 1) equals pcad_hidden_at_layers at s
+ * converted to fp32.
+ * The entries are read once, in the engine's own workspace, as each comes into existence; the only caller buffer is the
+ * result.  All 33 entries of PlantCaduceus_l32 at B = 256, L = 512 are 17.7 GB as pcad_forward_taps buffers and 69 MB
+ * pooled; all 49 of PlantCAD2-Large at B = 16, L = 8192 are 39.5 GB and 9.6 MB.  The workspace is that of any forward
+ * (pcad_workspace_bytes does not change).  Always stops at the deepest requested entry; never uses a CUDA graph.  Same
+ * argument checks as pcad_forward_taps, and PCAD_ERR_INVALID for a null out_dev, all before launching anything.  With
+ * B = 0 or L = 0 nothing is written. */
+#define PCAD_HIDDEN_MEAN_CHUNK 128
+int pcad_hidden_mean_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* ranges_dev, int B, int L,
+                               int n_taps, const int32_t* tap_idx, float* out_dev, void* stream);
+
 /* Token ids outside [0, vocab_size) (the reference's nn.Embedding would raise) are detected on the device by
  * pcad_forward / pcad_score_masked: the offending position is scored as id 0 and a flag is raised in mapped host
  * memory.  pcad_take_id_error returns PCAD_ERR_INVALID and clears the flag if any call since the last take saw such an
@@ -302,6 +327,13 @@ int pcad_op_ssd_scan(const void* xbc_f, const void* xbc_r, int64_t ld_xbc, const
  * out = rms(y_f * silu(z)) * w_f + rms(y_r * silu(z)) * w_r, rows of E channels; z has row pitch ldz. */
 int pcad_op_gated_norm_sum(const void* y_f, const void* y_r, const void* z, int64_t ldz, const float* w_f,
                            const float* w_r, void* out, int64_t rows, int E, float eps, int dtype, void* stream);
+
+/* The pooled mean of pcad_hidden_mean_at_layers for one entry, from the engine's strand-major rows: rows [2*B*L, d] (the
+ * B forward strands, then the B RC strands, each L rows of d channels; RC strand b's row t is position L-1-t of window b,
+ * channels reversed) -> out float32 [B, 2*d], with the same ranges, NaN rows and summation order.  scratch: float
+ * [B * ceil(L / PCAD_HIDDEN_MEAN_CHUNK) * 2 * d] (the chunk partials).  d a multiple of 8; rows 16-byte aligned. */
+int pcad_op_hidden_mean(const void* rows, const int32_t* ranges_dev, float* scratch, float* out, int B, int L, int d,
+                        int dtype, void* stream);
 
 #ifdef __cplusplus
 }

@@ -21,13 +21,13 @@ ABI_VERSION = 3
 EXPORTS = (
     "pcad_abi_version", "pcad_create", "pcad_destroy", "pcad_last_error", "pcad_set_weight", "pcad_finalize",
     "pcad_set_tokenizer", "pcad_take_id_error", "pcad_hidden_at", "pcad_forward",
-    "pcad_forward_taps", "pcad_hidden_at_layers", "pcad_score_masked", "pcad_score_masked_at", "pcad_score_windows_host", "pcad_score_windows_dev", "pcad_extract_windows", "pcad_tokenize",
+    "pcad_forward_taps", "pcad_hidden_at_layers", "pcad_hidden_mean_at_layers", "pcad_score_masked", "pcad_score_masked_at", "pcad_score_windows_host", "pcad_score_windows_dev", "pcad_extract_windows", "pcad_tokenize",
     "pcad_workspace_bytes", "pcad_set_profiling", "pcad_get_profile", "pcad_launch_count",
     "pcad_graph_replays",
     "pcad_op_linear", "pcad_op_linear_residual", "pcad_op_linear_residual_tap", "pcad_op_linear_rowscale", "pcad_op_sumsq_parts",
     "pcad_op_add_rmsnorm", "pcad_op_conv_silu", "pcad_op_biscan", "pcad_op_biscan_segmented", "pcad_op_biscan_ex",
     "pcad_op_biscan_dt",
-    "pcad_op_ssd_scan", "pcad_op_gated_norm_sum",
+    "pcad_op_ssd_scan", "pcad_op_gated_norm_sum", "pcad_op_hidden_mean",
 )
 
 
@@ -73,6 +73,7 @@ def load() -> C.CDLL:
     lib.pcad_forward.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.pcad_forward_taps.argtypes = [vp, vp, i32, i32, vp, i32, C.POINTER(C.c_int32), C.POINTER(vp), vp]
     lib.pcad_hidden_at_layers.argtypes = [vp, vp, vp, i32, i32, i32, i32, C.POINTER(C.c_int32), vp, vp]
+    lib.pcad_hidden_mean_at_layers.argtypes = [vp, vp, vp, i32, i32, i32, C.POINTER(C.c_int32), vp, vp]
     lib.pcad_score_masked.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
     lib.pcad_score_masked_at.argtypes = [vp, vp, i32, i32, i32, vp, vp]
     lib.pcad_score_windows_host.argtypes = [vp, vp, i32, i32, i32, vp, vp]
@@ -102,6 +103,7 @@ def load() -> C.CDLL:
                                       i32, i32, i32, i32, vp, vp, vp, i32, i32, vp]
     lib.pcad_op_ssd_scan.argtypes = [vp, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
     lib.pcad_op_gated_norm_sum.argtypes = [vp, vp, vp, i64, vp, vp, vp, i64, i32, C.c_float, i32, vp]
+    lib.pcad_op_hidden_mean.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp]
     for name in EXPORTS:
         getattr(lib, name)  # AttributeError here means header and library disagree
     if lib.pcad_abi_version() != ABI_VERSION:

@@ -433,4 +433,87 @@ __global__ void hidden_tap_pos_kernel(const T* __restrict__ H, const int* __rest
   store8<T>(out + item * (2 * d) + j0, x);
 }
 
+// ---- mean of a hidden_states entry over a range of positions (pcad_hidden_mean_at_layers, pcad_op_hidden_mean) ----
+// out[b, j] = mean over t in [s_b, e_b) of hidden_states[b, t, j] (the layout of hidden_tap_kernel), float32, with one
+// fixed summation order: fp32 sums of kHiddenMeanChunk consecutive positions counted from s_b, each sequential in t, then
+// the chunk partials summed sequentially in chunk order and divided by e_b - s_b (correctly rounded).  The order depends on
+// neither B nor any other window, and there are no atomics.  ranges: int32 [B, 2] or nullptr for [0, L).  An invalid range
+// (s < 0, e > L or s >= e) gives a NaN row.  part: float [B, ceil(L / kHiddenMeanChunk), 2d] scratch.
+constexpr int kHiddenMeanChunk = 128;
+
+__device__ __forceinline__ bool mean_range(const int* ranges, int b, int L, int& s, int& e) {
+  s = ranges ? ranges[2 * b] : 0;
+  e = ranges ? ranges[2 * b + 1] : L;
+  return s >= 0 && e <= L && s < e;
+}
+
+// Stage 1: one thread per (window, chunk, 8 output channels) sums its chunk's rows.  The RC half of position t is row
+// L-1-t of strand B+b with its channels reversed: the thread reads those rows in t order and reverses the 8 sums on store.
+template <typename T>
+__global__ void __launch_bounds__(128)
+hidden_mean_partial_kernel(const T* __restrict__ H, const int* __restrict__ ranges, float* __restrict__ part, int B, int L,
+                           int d, int n_chunks) {
+  const int vec_per_row = (2 * d) / 8;
+  const long long gid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (gid >= static_cast<long long>(B) * n_chunks * vec_per_row) return;
+  const int v = static_cast<int>(gid % vec_per_row);
+  const long long bc = gid / vec_per_row;
+  const int c = static_cast<int>(bc % n_chunks);
+  const int b = static_cast<int>(bc / n_chunks);
+  int s, e;
+  if (!mean_range(ranges, b, L, s, e)) return;
+  const int t0 = s + c * kHiddenMeanChunk;
+  if (t0 >= e) return;
+  const int n = min(kHiddenMeanChunk, e - t0);
+  const int j0 = v * 8;
+  const bool fwd = j0 < d;
+  const T* p = fwd ? H + (static_cast<long long>(b) * L + t0) * d + j0
+                   : H + (static_cast<long long>(B + b) * L + (L - 1 - t0)) * d + (2 * d - 8 - j0);
+  const long long step = fwd ? d : -static_cast<long long>(d);
+  float acc[8];
+  load8<T>(p, acc);
+#pragma unroll 8
+  for (int i = 1; i < n; ++i) {
+    float x[8];
+    load8<T>(p + i * step, x);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) acc[k] += x[k];
+  }
+  float o[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) o[k] = fwd ? acc[k] : acc[7 - k];
+  float4* q = reinterpret_cast<float4*>(part + bc * (2 * d) + j0);
+  q[0] = make_float4(o[0], o[1], o[2], o[3]);
+  q[1] = make_float4(o[4], o[5], o[6], o[7]);
+}
+
+// Stage 2: one thread per (window, output channel) sums that window's chunk partials in chunk order and divides.
+__global__ void __launch_bounds__(256)
+hidden_mean_final_kernel(const float* __restrict__ part, const int* __restrict__ ranges, float* __restrict__ out, int B,
+                         int L, int d, int n_chunks) {
+  const int w = 2 * d;
+  const long long gid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (gid >= static_cast<long long>(B) * w) return;
+  const int j = static_cast<int>(gid % w);
+  const int b = static_cast<int>(gid / w);
+  int s, e;
+  if (!mean_range(ranges, b, L, s, e)) {
+    out[gid] = __int_as_float(0x7fc00000);
+    return;
+  }
+  const int nc = (e - s + kHiddenMeanChunk - 1) / kHiddenMeanChunk;
+  const float* q = part + static_cast<long long>(b) * n_chunks * w + j;
+  float acc = q[0];
+  int c = 1;
+  for (; c + 8 <= nc; c += 8) {
+    float x[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) x[u] = q[static_cast<long long>(c + u) * w];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) acc += x[u];
+  }
+  for (; c < nc; ++c) acc += q[static_cast<long long>(c) * w];
+  out[gid] = __fdiv_rn(acc, static_cast<float>(e - s));
+}
+
 }  // namespace pcad

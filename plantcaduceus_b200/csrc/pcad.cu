@@ -504,6 +504,26 @@ int op_gated_norm_sum(pcad_handle* h, const void* y_f, const void* y_r, const vo
   return PCAD_OK;
 }
 
+static_assert(kHiddenMeanChunk == PCAD_HIDDEN_MEAN_CHUNK, "pcad.h states the chunk length of the pooled mean");
+
+// Mean over each window's range of one hidden_states entry held as strand-major [2BL, d] rows -> out float [B, 2d] (two
+// launches: chunk partials into `scratch`, float [B, ceil(L / kHiddenMeanChunk), 2d], then their sum in chunk order).
+int op_hidden_mean(pcad_handle* h, const void* rows, const int32_t* ranges, float* scratch, float* out, int B, int L, int d,
+                   bool f32, cudaStream_t st) {
+  if (d <= 0 || d % 8) return fail(h, PCAD_ERR_INVALID, "hidden_mean: d must be a positive multiple of 8");
+  if (B < 0 || L < 0) return fail(h, PCAD_ERR_INVALID, "hidden_mean: negative batch or length");
+  if (B == 0 || L == 0) return PCAD_OK;
+  const int n_chunks = (L + kHiddenMeanChunk - 1) / kHiddenMeanChunk;
+  const long long items = static_cast<long long>(B) * n_chunks * (2 * d / 8);
+  const unsigned blocks1 = static_cast<unsigned>((items + 127) / 128);
+  if (f32) hidden_mean_partial_kernel<float><<<blocks1, 128, 0, st>>>(static_cast<const float*>(rows), ranges, scratch, B, L, d, n_chunks);
+  else hidden_mean_partial_kernel<bf16><<<blocks1, 128, 0, st>>>(static_cast<const bf16*>(rows), ranges, scratch, B, L, d, n_chunks);
+  const unsigned blocks2 = static_cast<unsigned>((static_cast<long long>(B) * 2 * d + 255) / 256);
+  hidden_mean_final_kernel<<<blocks2, 256, 0, st>>>(scratch, ranges, out, B, L, d, n_chunks);
+  CUDA_TRY(h, cudaGetLastError());
+  return PCAD_OK;
+}
+
 // ws.xz holds in_proj's output [T, DIPP]: z at [0, E), x|B|C at [E, E + CD), dt at [E + CD, E + CD + H).  Leaves the summed,
 // normed y in ws.y.  [EXT mamba_ssm Mamba2.forward, non-fused branch; BiMambaWrapper "add" with tied projections]
 int run_mixer_m2(pcad_handle* h, LayerWeights& lw, int S, int L, cudaStream_t st) {
@@ -607,13 +627,16 @@ __global__ void gather_rows_kernel(const uint4* __restrict__ src, uint4* __restr
 
 // ---- hidden-state taps ---------------------------------------------------------------------------------
 // Which entries of the reference's hidden_states tuple a forward emits, and where: idx[i] (strictly increasing, in
-// [0, n_layer]) goes to dst[i], [B, L, 2d] in the model dtype; or, with pos, [B, n_pos, 2d] at the positions pos[b, :].
+// [0, n_layer]) goes to dst[i], [B, L, 2d] in the model dtype; or, with pos, [B, n_pos, 2d] at the positions pos[b, :];
+// or, with mean, float [B, 2d] at mean + i * B * 2d: the mean over each window's range (op_hidden_mean).
 struct Taps {
   int n = 0;
   const int32_t* idx = nullptr;
   void* const* dst = nullptr;
   const int32_t* pos = nullptr;   // device, [B, n_pos]; nullptr: every position
   int n_pos = 0;
+  float* mean = nullptr;          // device, [n, B, 2d]: pooled mode (dst and pos unused)
+  const int32_t* ranges = nullptr;   // device, [B, 2] for the pooled mode; nullptr: [0, L) for every window
   int deepest() const { return n > 0 ? idx[n - 1] : -1; }
   int find(int k) const {   // i with idx[i] == k, or -1
     for (int i = 0; i < n; ++i)
@@ -623,12 +646,18 @@ struct Taps {
 };
 
 // Writes hidden_states[k] from the strand-major [2BL, d] rows `src` into dst[i] if k is tap i (hidden_tap_kernel /
-// hidden_tap_pos_kernel: the RC half reversed in time and channels).
+// hidden_tap_pos_kernel: the RC half reversed in time and channels), or its per-window mean in the pooled mode.
 int emit_tap(pcad_handle* h, const Taps* taps, int k, const void* src, int B, int L, cudaStream_t st) {
   const int i = taps ? taps->find(k) : -1;
   if (i < 0) return PCAD_OK;
-  StageTimer tm(h, st, PCAD_ST_MISC);
+  StageTimer tm(h, st, PCAD_ST_MISC, taps->mean ? 2 : 1);
   const int d = h->d;
+  if (taps->mean) {
+    // the partials, 2B ceil(L / P) d floats, go to ws.delta[0] ([T, E] with E = 2d, so they fit): the scan has consumed it
+    // whenever a tap is emitted, and the pruned last layer that reuses it never runs with taps
+    return op_hidden_mean(h, src, taps->ranges, static_cast<float*>(h->ws.delta[0]), taps->mean + static_cast<size_t>(i) * B * 2 * d,
+                          B, L, d, h->f32, st);
+  }
   if (taps->pos) {
     const long long total = static_cast<long long>(B) * taps->n_pos * (2 * d / 8);
     const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
@@ -1395,6 +1424,25 @@ int pcad_hidden_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t*
   return run_backbone(h, B, L, st, -1, &taps, false);
 }
 
+int pcad_hidden_mean_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* ranges_dev, int B, int L, int n_taps,
+                               const int32_t* tap_idx, float* out_dev, void* stream) {
+  if (!h) return PCAD_ERR_INVALID;
+  int rc = check_taps(h, n_taps, tap_idx);
+  if (rc) return rc;
+  if (!out_dev) return fail(h, PCAD_ERR_INVALID, "out_dev is null");
+  rc = begin_call(h, B, L, 1, ids_dev != nullptr, "ids_dev is null");
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = stage_ids(h, ids_dev, B, L, -1, st);
+  if (rc) return rc;
+  Taps taps;
+  taps.n = n_taps;
+  taps.idx = tap_idx;
+  taps.mean = out_dev;
+  taps.ranges = ranges_dev;
+  return run_backbone(h, B, L, st, -1, &taps, false);
+}
+
 int pcad_score_windows_host(pcad_handle* h, const uint8_t* ascii_host, int B, int L, int token_idx, float* logits4_host, void* stream) {
   int rc = begin_call(h, B, L, 1, ascii_host && logits4_host, "null argument", token_idx);
   if (rc) return rc == kNoWork ? PCAD_OK : rc;
@@ -1570,6 +1618,13 @@ int pcad_op_gated_norm_sum(const void* y_f, const void* y_r, const void* z, int6
   if (dtype != PCAD_BF16 && dtype != PCAD_F32) return PCAD_ERR_INVALID;
   return op_fail_to_global(op_gated_norm_sum(op_scratch(), y_f, y_r, z, ldz, w_f, w_r, out, rows, E, eps, dtype == PCAD_F32,
                                              static_cast<cudaStream_t>(stream)));
+}
+
+int pcad_op_hidden_mean(const void* rows, const int32_t* ranges_dev, float* scratch, float* out, int B, int L, int d, int dtype,
+                        void* stream) {
+  if ((dtype != PCAD_BF16 && dtype != PCAD_F32) || !rows || !scratch || !out) return PCAD_ERR_INVALID;
+  return op_fail_to_global(op_hidden_mean(op_scratch(), rows, ranges_dev, scratch, out, B, L, d, dtype == PCAD_F32,
+                                          static_cast<cudaStream_t>(stream)));
 }
 
 }  // extern "C"

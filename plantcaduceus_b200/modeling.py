@@ -64,6 +64,21 @@ def hidden_layer_indices(layers: Union[str, Iterable[int]], n_layer: int) -> Lis
     return out
 
 
+def hidden_mean_ranges(ranges, B: int, L: int) -> torch.Tensor:
+    """Per-window ranges [s_b, e_b) for ``hidden_mean`` as int32 [B, 2] (on ``ranges``' device).  Raises ValueError unless
+    ``ranges`` is [B, 2] integers (a tensor, an array or nested sequences).  Values are clamped to [-1, L + 1], which keeps
+    every valid range and keeps every invalid one invalid, so that no int64 value wraps into a valid int32 range."""
+    try:
+        r = ranges if isinstance(ranges, torch.Tensor) else torch.as_tensor(np.asarray(ranges))
+    except (TypeError, ValueError, RuntimeError) as e:
+        raise ValueError(f"ranges must be [B, 2] integers: {e}") from None
+    if r.dtype not in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8):
+        raise ValueError(f"ranges must be [B, 2] integers, not {r.dtype}")
+    if tuple(r.shape) != (B, 2):
+        raise ValueError(f"ranges must be [B, 2] = [{B}, 2], not {list(r.shape)}")
+    return r.to(torch.int64).clamp(-1, L + 1).to(torch.int32).contiguous()
+
+
 class CaduceusForMaskedLM:
     """Inference-only Caduceus masked LM backed by libpcad."""
 
@@ -362,6 +377,35 @@ class CaduceusForMaskedLM:
             if want != layers:   # the engine takes the indices in increasing order; return them in the caller's
                 out = out[torch.tensor([want.index(k) for k in layers], device=self.device)]
         return out
+
+    def hidden_mean(self, ids_u8: torch.Tensor, ranges=None, layers: Union[None, str, Iterable[int]] = None) -> torch.Tensor:
+        """Mean over each window's positions of a ``hidden_states`` entry, float32, without [B, L, 2*d_model] buffers:
+        ``out[b] = hidden_states[k][b, s_b:e_b].float().mean(0)`` in the engine's fixed summation order (pcad.h,
+        pcad_hidden_mean_at_layers).  ``ranges``: [B, 2] integers (s_b, e_b), or None for every position; a window whose
+        range is invalid (s < 0, e > L or s >= e) gets a NaN row.  ``layers=None``: [B, 2*d_model] from the final normed
+        state; otherwise ("all", or indices as ``forward``'s ``hidden_layers``) [len(layers), B, 2*d_model] in the caller's
+        order.  The forward stops after the deepest requested layer.  Raises ValueError for ranges that are not [B, 2]
+        integers."""
+        self._require_handle()
+        final = layers is None
+        want_layers = [self.config.n_layer] if final else hidden_layer_indices(layers, self.config.n_layer)
+        ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
+        B, L = ids.shape
+        rng = None if ranges is None else hidden_mean_ranges(ranges, B, L).to(self.device)
+        want = sorted(want_layers)
+        with torch.cuda.device(self.device):
+            out = torch.empty((len(want), B, 2 * self.config.d_model), dtype=torch.float32, device=self.device)
+            if B > 0 and L > 0:
+                idx = (C.c_int32 * len(want))(*want)
+                _lib.check(self._lib.pcad_hidden_mean_at_layers(
+                    self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(rng.data_ptr()) if rng is not None else None, B, L,
+                    len(want), idx, C.c_void_p(out.data_ptr()), self._stream()), self._handle)
+                self._raise_on_bad_ids(True)
+            else:
+                out.fill_(float("nan"))   # L = 0: no range is valid
+            if want != want_layers:   # the engine takes the indices in increasing order; return them in the caller's
+                out = out[torch.tensor([want.index(k) for k in want_layers], device=self.device)]
+        return out[0] if final else out
 
     def score_windows_host(self, ascii_windows: Union[np.ndarray, torch.Tensor], token_idx: int,
                            out: Optional[torch.Tensor] = None) -> torch.Tensor:
