@@ -302,16 +302,6 @@ int pcad_op_biscan_ex(const void* u_f, const void* delta_f, const void* bc_f,
                       void* y, int S, int L, int E, int segments, float* seg_state, float* seg_sumd,
                       float* bc_rows, int Lrun, int dtype, void* stream);
 
-/* The same with Mamba.dt_proj [F.linear(dt, dt_proj.weight)] computed inside the scan kernel on the tensor core (bf16 only):
- * dbc_* are the x_proj outputs [S*L, ldbc] (dt in columns [0, R), B at [bc_off, bc_off+16), C at [bc_off+16, bc_off+32);
- * ldbc >= 64), wdt_* the dt_proj weights [E, R] with row pitch ldw (elements, a multiple of 8; R <= 64).  Delta is rounded
- * to bf16 where the GEMM would have rounded it, so the result matches pcad_op_linear + pcad_op_biscan. */
-int pcad_op_biscan_dt(const void* u_f, const void* dbc_f, const void* u_r, const void* dbc_r, int64_t ldbc, int bc_off,
-                      const void* wdt_f, const void* wdt_r, int64_t ldw, int R, const void* z, int64_t ldz,
-                      const float* A_f, const float* D_f, const float* dt_bias_f,
-                      const float* A_r, const float* D_r, const float* dt_bias_r,
-                      void* y, int S, int L, int E, void* stream);
-
 /* Mamba-2 / SSD selective scan [mamba_chunk_scan_combined(x, dt, A, B, C, D=D, z=None, dt_bias, dt_softplus=True)] for
  * both time directions (direction by index math): xbc_f / xbc_r are the two directions' conv + SiLU outputs
  * [S*L, ld_xbc] with x at columns [0, 64 H), B at [64 H, 64 H + 64), C at [64 H + 64, 64 H + 128) (64-wide heads, 64

@@ -26,7 +26,6 @@ EXPORTS = (
     "pcad_graph_replays",
     "pcad_op_linear", "pcad_op_linear_residual", "pcad_op_linear_residual_tap", "pcad_op_linear_rowscale", "pcad_op_sumsq_parts",
     "pcad_op_add_rmsnorm", "pcad_op_conv_silu", "pcad_op_biscan", "pcad_op_biscan_segmented", "pcad_op_biscan_ex",
-    "pcad_op_biscan_dt",
     "pcad_op_ssd_scan", "pcad_op_gated_norm_sum", "pcad_op_hidden_mean",
 )
 
@@ -94,7 +93,6 @@ def load() -> C.CDLL:
     lib.pcad_op_sumsq_parts.argtypes = [i32]
     lib.pcad_op_add_rmsnorm.argtypes = [vp, vp, vp, vp, vp, i64, i32, C.c_float, i32, i32, vp]
     lib.pcad_op_conv_silu.argtypes = [vp, i64, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
-    lib.pcad_op_biscan_dt.argtypes = [vp, vp, vp, vp, i64, i32, vp, vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]
     lib.pcad_op_biscan.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp,
                                    i32, i32, i32, i32, vp]
     lib.pcad_op_biscan_segmented.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp,

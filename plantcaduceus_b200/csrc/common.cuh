@@ -339,30 +339,6 @@ __device__ __forceinline__ void umma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, u
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// ksteps (1..4) K = 16 steps of one 64-wide K block (128-byte swizzled K-major operands: +32 bytes per step) into a fresh
-// accumulator, then the commit -- ONE asm statement, so the compiler moves the operands to uniform registers once instead of
-// once per instruction (the issuing thread of the scan kernel is a compute thread: every instruction here is on its
-// critical path).
-__device__ __forceinline__ void umma_bf16_ss_k64_commit(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                        int ksteps, uint64_t* bar) {
-  asm volatile(
-      "{\n\t.reg .pred pz, po, p1, p2, p3;\n\t.reg .b64 a1, b1, a2, b2, a3, b3;\n\t"
-      "setp.ne.b32 pz, 0, 0;\n\t"
-      "setp.eq.b32 po, 0, 0;\n\t"
-      "setp.gt.s32 p1, %4, 1;\n\t"
-      "setp.gt.s32 p2, %4, 2;\n\t"
-      "setp.gt.s32 p3, %4, 3;\n\t"
-      "add.s64 a1, %1, 2;\n\tadd.s64 b1, %2, 2;\n\t"
-      "add.s64 a2, %1, 4;\n\tadd.s64 b2, %2, 4;\n\t"
-      "add.s64 a3, %1, 6;\n\tadd.s64 b3, %2, 6;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, pz;\n\t"
-      "@p1 tcgen05.mma.cta_group::1.kind::f16 [%0], a1, b1, %3, po;\n\t"
-      "@p2 tcgen05.mma.cta_group::1.kind::f16 [%0], a2, b2, %3, po;\n\t"
-      "@p3 tcgen05.mma.cta_group::1.kind::f16 [%0], a3, b3, %3, po;\n\t"
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%5];\n\t}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(ksteps), "r"(smem_u32(bar))
-      : "memory");
-}
 // Arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar))
@@ -390,12 +366,6 @@ __device__ __forceinline__ void tmem_ld_32x32b_x16(uint32_t taddr, uint32_t (&r)
         "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
       : "r"(taddr)
       : "memory");
-}
-// TMEM -> register: this warp's 32 lanes x 1 fp32 column.
-__device__ __forceinline__ uint32_t tmem_ld_32x32b_x1(uint32_t taddr) {
-  uint32_t r;
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\n" : "=r"(r) : "r"(taddr) : "memory");
-  return r;
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
 

@@ -79,7 +79,6 @@ struct pcad_handle {
   int ssd_impl = 0;                    // Mamba-2 bf16 A/B switch: 0 chunked SSD on tcgen05, 1 sequential recurrence
   int H = 0, CD = 0, DIP = 0, DIPP = 0;   // Mamba-2: heads, conv channels (x|B|C), in_proj width (z|x|B|C|dt) and its padded pitch
   bool f32 = false;
-  bool fuse_dt = false;                // bf16: dt_proj computed inside the scan (tcgen05), no dt_proj launches, no delta in HBM
   bool bc_f32 = true;                  // bf16: B|C converted to fp32 rows once (bc_to_f32_kernel), scan in its one-barrier mode
   bool bc_f32_force = false;           // ... also below the size where it pays (tests)
   bool fuse_norm = false;   // bf16 activations + bf16 residual: add+RMSNorm folded into the out_proj / in_proj epilogues
@@ -326,8 +325,7 @@ int op_conv(pcad_handle* h, const void* x, long long ldx, const float* w_f, cons
 int op_biscan(pcad_handle* h, const void* u_f, const void* delta_f, const void* bc_f, const void* u_r,
               const void* delta_r, const void* bc_r, long long ldbc, int bc_off, const void* z, long long ldz,
               const float* A_f, const float* D_f, const float* bias_f, const float* A_r, const float* D_r,
-              const float* bias_r, void* y, int S, int L, int E, bool f32, cudaStream_t st,
-              const void* wdt_f = nullptr, const void* wdt_r = nullptr, long long ldw = 0, int R = 0, int segments = 1,
+              const float* bias_r, void* y, int S, int L, int E, bool f32, cudaStream_t st, int segments = 1,
               float* seg_state = nullptr, float* seg_sumd = nullptr, int Lrun = 0, float* bcf = nullptr) {
   const int vec = f32 ? 4 : 8;
   if (E % vec || ldbc % vec || bc_off % vec || ldz % vec)
@@ -335,8 +333,7 @@ int op_biscan(pcad_handle* h, const void* u_f, const void* delta_f, const void* 
   if (S <= 0 || L <= 0) return PCAD_OK;
   if (S > 65535) return fail(h, PCAD_ERR_INVALID, "biscan: at most 65535 sequences per call");
   // rejected before anything is launched: these combinations used to be accepted with one argument silently ignored
-  if (bcf && (f32 || wdt_f || wdt_r))
-    return fail(h, PCAD_ERR_INVALID, "biscan: fp32 B|C rows are a mode of the bf16 scan without the in-kernel dt_proj");
+  if (bcf && f32) return fail(h, PCAD_ERR_INVALID, "biscan: fp32 B|C rows are a mode of the bf16 scan");
   if (Lrun < 0 || Lrun > L || (Lrun > 0 && Lrun < (L + 1) / 2))
     return fail(h, PCAD_ERR_INVALID, "biscan: Lrun = %d must be 0 or in [(L+1)/2, L] = [%d, %d] (below, some rows are visited by neither direction)",
                 Lrun, (L + 1) / 2, L);
@@ -347,11 +344,10 @@ int op_biscan(pcad_handle* h, const void* u_f, const void* delta_f, const void* 
   static_cast<const TT*>(u_f), static_cast<const TT*>(delta_f), static_cast<const TT*>(bc_f), static_cast<const TT*>(u_r), \
       static_cast<const TT*>(delta_r), static_cast<const TT*>(bc_r), ldbc, bc_off, static_cast<const TT*>(z), ldz, A_f, D_f, \
       bias_f, A_r, D_r, bias_r, static_cast<TT*>(y), S, L, E
-  const bool fused_dt = wdt_f != nullptr || wdt_r != nullptr;
-  // bcf (bf16, not fused): scratch for float [2][S*L][32]; B|C are converted once here and the scan runs its one-barrier mode
+  // bcf (bf16): scratch for float [2][S*L][32]; B|C are converted once here and the scan runs its one-barrier mode
   const float* bcf_f = nullptr;
   const float* bcf_r = nullptr;
-  if (bcf && !f32 && !fused_dt) {
+  if (bcf) {
     const long long rows = static_cast<long long>(S) * L;
     bc_to_f32_kernel<<<static_cast<unsigned>((rows * 8 + 255) / 256), 256, 0, st>>>(static_cast<const bf16*>(bc_f), static_cast<const bf16*>(bc_r),
                                                                                   ldbc, bc_off, bcf, rows);
@@ -360,24 +356,19 @@ int op_biscan(pcad_handle* h, const void* u_f, const void* delta_f, const void* 
     bcf_r = bcf + rows * 2 * kScanN;
   }
   if (segments > 1) {   // time-parallel: `segments` concurrent segments per sequence (scan.cuh)
-    if (fused_dt || !seg_state || !seg_sumd || L % segments || static_cast<long long>(S) * segments > 65535)
+    if (!seg_state || !seg_sumd || L % segments || static_cast<long long>(S) * segments > 65535)
       return fail(h, PCAD_ERR_INVALID, "biscan: the time-parallel scan needs L %% segments == 0, S * segments <= 65535 and its state buffers");
     if (f32) e = launch_biscan_time_parallel<float, true>(PCAD_SCAN_ARGS(float), segments, seg_state, seg_sumd, st);
     else e = launch_biscan_time_parallel<bf16, false>(PCAD_SCAN_ARGS(bf16), segments, seg_state, seg_sumd, st, bcf_f, bcf_r);
     CUDA_TRY(h, e);
     return PCAD_OK;
   }
-  if (fused_dt) {   // delta_* are the x_proj outputs, dt_proj runs inside the kernel (tcgen05)
-    if (f32 || !wdt_f || !wdt_r || ldbc < kScanDtK || R <= 0 || R > kScanDtK || ldw < R || ldw % 8)
-      return fail(h, PCAD_ERR_INVALID, "biscan: the in-kernel dt_proj needs bf16, both weights (R <= 64, row pitch a multiple of 8) and ldbc >= 64");
-    e = launch_biscan<bf16, false, kScanFusedDt>(PCAD_SCAN_ARGS(bf16), st, static_cast<const bf16*>(wdt_f), static_cast<const bf16*>(wdt_r),
-                                                 ldw, R, nullptr, Lrun);
-  } else if (f32) {
-    e = launch_biscan<float, true, kScanPlain>(PCAD_SCAN_ARGS(float), st, nullptr, nullptr, 0, 0, nullptr, Lrun);
+  if (f32) {
+    e = launch_biscan<float, true, kScanPlain>(PCAD_SCAN_ARGS(float), st, nullptr, Lrun);
   } else if (bcf_f) {
-    e = launch_biscan<bf16, false, kScanBcF32>(PCAD_SCAN_ARGS(bf16), st, nullptr, nullptr, 0, 0, nullptr, Lrun, bcf_f, bcf_r);
+    e = launch_biscan<bf16, false, kScanBcF32>(PCAD_SCAN_ARGS(bf16), st, nullptr, Lrun, bcf_f, bcf_r);
   } else {
-    e = launch_biscan<bf16, false, kScanPlain>(PCAD_SCAN_ARGS(bf16), st, nullptr, nullptr, 0, 0, nullptr, Lrun);
+    e = launch_biscan<bf16, false, kScanPlain>(PCAD_SCAN_ARGS(bf16), st, nullptr, Lrun);
   }
 #undef PCAD_SCAN_ARGS
   CUDA_TRY(h, e);
@@ -582,15 +573,13 @@ int run_mixer_m1(pcad_handle* h, LayerWeights& lw, int S, int L, int prune_idx, 
     if (rc) return rc;
   }
   const int P = scan_segments(h, S, L);
-  // dt_proj runs inside the scan kernel (tcgen05, scan.cuh) unless the time-parallel passes need delta in memory
-  const bool fuse_dt = h->fuse_dt && P == 1;
   for (int dir = 0; dir < 2; ++dir) {
     {
       StageTimer tm(h, st, PCAD_ST_X_PROJ);
       rc = op_linear(h, ws.xc[dir], lw.dir[dir].x_proj, ws.dbc[dir], T, RP, E, E, E, RP, f32, h->num_sms, st);
       if (rc) return rc;
     }
-    if (!fuse_dt) {
+    {
       StageTimer tm(h, st, PCAD_ST_DT_PROJ);
       rc = op_linear(h, ws.dbc[dir], lw.dir[dir].dt_proj, ws.delta[dir], T, E, R, RP, R, E, f32, h->num_sms, st);
       if (rc) return rc;
@@ -603,13 +592,9 @@ int run_mixer_m1(pcad_handle* h, LayerWeights& lw, int S, int L, int prune_idx, 
   // fp32 B|C rows + one-barrier scan mode: one more (tiny) launch per layer, so only where the scan is long enough to
   // repay it (measured: -1 ms of 170 per step at T = 262 144; launch-bound small batches keep the in-kernel conversion)
   const bool use_bcf = h->bc_f32 && !f32 && (h->bc_f32_force || T >= 65536);
-  if (fuse_dt)   // the scan reads the x_proj outputs (dt | B | C) and the dt_proj weights
-    return op_biscan(h, ws.xc[0], ws.dbc[0], ws.dbc[0], ws.xc[1], ws.dbc[1], ws.dbc[1], RP, R, zbase, 2 * E,
-                     lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32,
-                     st, lw.dir[0].dt_proj, lw.dir[1].dt_proj, R, R, 1, nullptr, nullptr, Lrun);
   rc = op_biscan(h, ws.xc[0], ws.delta[0], ws.dbc[0], ws.xc[1], ws.delta[1], ws.dbc[1], RP, R, zbase, 2 * E,
                  lw.dir[0].A, lw.dir[0].D, lw.dir[0].dt_bias, lw.dir[1].A, lw.dir[1].D, lw.dir[1].dt_bias, ws.y, S, L, E, f32, st,
-                 nullptr, nullptr, 0, 0, P, ws.seg_state, ws.seg_sumd, Lrun, use_bcf ? ws.bcf : nullptr);
+                 P, ws.seg_state, ws.seg_sumd, Lrun, use_bcf ? ws.bcf : nullptr);
   if (P > 1) h->launch_count += 2;
   if (use_bcf) h->launch_count += 1;
   return rc;
@@ -948,11 +933,6 @@ int pcad_create(const pcad_config* cfg, int device, pcad_handle** out) {
   h->f32 = cfg->dtype == PCAD_F32;
   h->act_size = h->f32 ? 4 : 2;
   h->fuse_norm = !h->f32 && !cfg->residual_in_fp32;
-  // dt_proj inside the scan kernel (bf16; x_proj output rows must hold at least 64 columns for the TMA box).
-  // Off by default: measured slower on B200 (scan +21 ms, dt_proj -12 ms per step; see scan.cuh).
-  h->fuse_dt = false;
-  if (const char* fd = getenv("PCAD_FUSED_DT"))
-    h->fuse_dt = fd[0] == '1' && !m2 && !h->f32 && h->RP >= kScanDtK && h->R <= kScanDtK && (h->E % 8) == 0;
   if (const char* bq = getenv("PCAD_SCAN_BC_F32")) { h->bc_f32 = bq[0] != '0'; h->bc_f32_force = bq[0] == '1'; }   // A/B switch: 0 off, 1 always
   if (const char* pl = getenv("PCAD_NO_PRUNE")) h->prune_last = pl[0] != '1';
   if (const char* tp = getenv("PCAD_NO_TIME_PARALLEL")) h->time_parallel = tp[0] != '1';
@@ -1557,15 +1537,6 @@ int pcad_op_linear_rowscale(const void* A, const void* W, const float* sumsq_in,
   return op_fail_to_global(op_linear(op_scratch(), A, W, C, M, N, K, lda, ldw, ldc, false, op_num_sms(), static_cast<cudaStream_t>(stream), kEpiRowScale, ep));
 }
 
-int pcad_op_biscan_dt(const void* u_f, const void* dbc_f, const void* u_r, const void* dbc_r, int64_t ldbc, int bc_off,
-                      const void* wdt_f, const void* wdt_r, int64_t ldw, int R, const void* z, int64_t ldz, const float* A_f,
-                      const float* D_f, const float* dt_bias_f, const float* A_r, const float* D_r, const float* dt_bias_r, void* y,
-                      int S, int L, int E, void* stream) {
-  if (!wdt_f || !wdt_r) return PCAD_ERR_INVALID;
-  return op_fail_to_global(op_biscan(op_scratch(), u_f, dbc_f, dbc_f, u_r, dbc_r, dbc_r, ldbc, bc_off, z, ldz, A_f, D_f, dt_bias_f,
-                                     A_r, D_r, dt_bias_r, y, S, L, E, false, static_cast<cudaStream_t>(stream), wdt_f, wdt_r, ldw, R));
-}
-
 int pcad_op_add_rmsnorm(const void* x, const void* res_in, const float* w, void* y, void* res_out, int64_t rows, int d, float eps, int dtype, int res_dtype, void* stream) {
   if (dtype != PCAD_BF16 && dtype != PCAD_F32) return PCAD_ERR_INVALID;
   if (dtype == PCAD_F32 && res_dtype != PCAD_F32) return PCAD_ERR_INVALID;
@@ -1591,8 +1562,8 @@ int pcad_op_biscan_segmented(const void* u_f, const void* delta_f, const void* b
                              float* seg_state, float* seg_sumd, int dtype, void* stream) {
   if (dtype != PCAD_BF16 && dtype != PCAD_F32) return PCAD_ERR_INVALID;
   return op_fail_to_global(op_biscan(op_scratch(), u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, dt_bias_f,
-                                     A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream), nullptr,
-                                     nullptr, 0, 0, segments, seg_state, seg_sumd));
+                                     A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream), segments,
+                                     seg_state, seg_sumd));
 }
 
 int pcad_op_biscan_ex(const void* u_f, const void* delta_f, const void* bc_f, const void* u_r, const void* delta_r, const void* bc_r,
@@ -1601,8 +1572,8 @@ int pcad_op_biscan_ex(const void* u_f, const void* delta_f, const void* bc_f, co
                       float* seg_state, float* seg_sumd, float* bc_rows, int Lrun, int dtype, void* stream) {
   if (dtype != PCAD_BF16 && dtype != PCAD_F32) return PCAD_ERR_INVALID;
   return op_fail_to_global(op_biscan(op_scratch(), u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, dt_bias_f,
-                                     A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream), nullptr,
-                                     nullptr, 0, 0, segments < 1 ? 1 : segments, seg_state, seg_sumd, Lrun, bc_rows));
+                                     A_r, D_r, dt_bias_r, y, S, L, E, dtype == PCAD_F32, static_cast<cudaStream_t>(stream),
+                                     segments < 1 ? 1 : segments, seg_state, seg_sumd, Lrun, bc_rows));
 }
 
 int pcad_op_ssd_scan(const void* xbc_f, const void* xbc_r, int64_t ld_xbc, const void* dt_raw, int64_t ld_dt, const float* A_f,

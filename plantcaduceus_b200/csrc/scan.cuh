@@ -15,7 +15,7 @@
 // Step i advances the forward scan at t_f = i and the reverse scan at t_r = L-1-i.  Inputs are streamed in chunks
 // of 16 steps by TMA (3-D tensor maps, one elected lane, 2-stage mbarrier ring: see biscan_kernel); the 32 B/C
 // values per step arrive as fp32 rows (kScanBcF32: converted once per layer by bc_to_f32_kernel) or are converted to fp32
-// once per chunk (kScanPlain, kScanFusedDt) and are broadcast-read.  Each thread leaves its un-gated y for
+// once per chunk (kScanPlain) and are broadcast-read.  Each thread leaves its un-gated y for
 // the chunk in shared memory; a vectorised chunk epilogue then either parks the partial in y (the other direction
 // has not reached that position yet) or adds the other direction's parked partial, applies SiLU(z) and stores the
 // final value -- 16-byte global accesses only.
@@ -33,8 +33,7 @@
 //     loop disappear);
 // (e) every instruction outside the main loop counts (the kernel issues at ~0.65 IPC): loads are TMA issued behind
 //     elect.sync (the six UTMALDG back to back), the forward's mode has no B|C conversion pass and ONE block barrier per
-//     chunk, the epilogue and the prefetch of parked partials have branch-free block-uniform fast paths;
-// (f) optionally (kScanFusedDt) dt_proj itself runs in the kernel on tcgen05, delta going TMEM -> registers.
+//     chunk, the epilogue and the prefetch of parked partials have branch-free block-uniform fast paths.
 // Built, measured and removed (profiles/r01_scan_step_ub.txt): FMA-pipe polynomial exponentials for part of the 8 pairs
 // (packed FFMA2 with three distinct operands runs at ~2.7 cycles, so a polynomial pair costs more issue/FMA time than the
 // MUFU time it frees: 5.11 / 5.33 ms with 1 / 2 of 8 pairs against 5.08), whole-warp polynomial flavours, a
@@ -75,29 +74,18 @@ constexpr int kScanUnroll = PCAD_SCAN_UNROLL;   // steps per main-loop block (st
 
 template <int V> struct IntTag { static constexpr int value = V; };
 
-constexpr int kScanDtK = 64;        // FUSEDT: contraction length of the in-kernel dt_proj (dt_rank zero-padded to 64 by the TMA)
-constexpr int kScanTmemCols = 64;   // FUSEDT: 2 stages x 32 fp32 columns (16 forward steps | 16 reverse-box rows)
-
-// Kernel modes.
+// Kernel modes (the values are part of the kernel names that profiles/ and tools/summarize_profiles.py quote).
 //   kScanPlain: delta arrives ready-made (dt_proj ran as a GEMM), B|C arrive as activations and are converted to fp32 in the
 //     kernel, once per chunk, behind a block barrier (the fp32 parity path and the operator API).
 //   kScanBcF32 (bf16, what the forward runs): B|C arrive as fp32 rows (B already scaled by ln 2: bc_to_f32_kernel), delivered by
 //     TMA like everything else -- no conversion pass, and with the chunk outputs double-buffered ONE block barrier per chunk.
-//   kScanFusedDt (bf16): the stage carries the rank-R dt rows of the x_proj outputs instead of delta -- one [32][64] tile (16
-//     forward rows, then the reverse box's 16 rows), 128-byte swizzled by TMA: the B operand of a tcgen05.mma whose A operand is
-//     this block's slice of dt_proj.weight.
-constexpr int kScanPlain = 0, kScanFusedDt = 1, kScanBcF32 = 2;
+constexpr int kScanPlain = 0, kScanBcF32 = 2;
 template <typename T, int MODE> struct ScanStage;
 template <typename T>
 struct ScanStage<T, kScanPlain> {
   T u[2][kScanTC][kScanCH];          // [direction][step][channel]
   T d[2][kScanTC][kScanCH];
   T bc_raw[2][kScanTC][2 * kScanN];
-};
-template <typename T>
-struct ScanStage<T, kScanFusedDt> {
-  T dt[2][kScanTC][kScanDtK];        // x_proj output columns 0..63 (dt | whatever follows: the zero-filled weight columns cancel it)
-  T u[2][kScanTC][kScanCH];
 };
 template <typename T>
 struct ScanStage<T, kScanBcF32> {
@@ -112,14 +100,6 @@ struct ScanShared<T, kScanPlain> {
   ScanStage<T, kScanPlain> st[2];
   float bc[2][kScanTC][2 * kScanN];   // fp32 B|C of the chunk being computed
   T pz[2][2][kScanTC][kScanCH];       // [partial | z][direction][step][channel]: prefetched for the chunk epilogue
-};
-template <typename T>
-struct ScanShared<T, kScanFusedDt> {
-  T wdt[2][kScanCH][kScanDtK];        // dt_proj.weight rows of this block's channels, forward then reverse: 128 x 64, swizzled
-  ScanStage<T, kScanFusedDt> st[2];
-  T bc_raw[2][kScanTC][2 * kScanN];   // single-buffered: consumed (converted to fp32) before the next chunk's loads are issued
-  float bc[2][kScanTC][2 * kScanN];
-  T pz[2][2][kScanTC][kScanCH];
 };
 template <typename T>
 struct ScanShared<T, kScanBcF32> {
@@ -247,31 +227,19 @@ template <> struct ScanDir<false> {
 // either direction) are zero-filled by the hardware.  The reverse direction's box holds ascending rows
 // L-16(c+1) .. L-16c-1, i.e. step j of the chunk sits in box row 15-j.  The parked partials and z rows that the
 // chunk epilogue needs are fetched with cp.async (generic proxy: they were written by this CTA's own st.global).
-//
-// FUSEDT (bf16): dt_proj [EXT Mamba.dt_proj, F.linear(dt, W)] runs inside the scan on the tensor core, so the two dt_proj
-// launches of a layer and the 4 KB per token of delta they write and the scan re-reads disappear.  tm_df / tm_dr map the
-// x_proj outputs (columns 0..63, 128-byte swizzle) instead of delta; tm_wf / tm_wr map dt_proj.weight [E, R] (box 64 x 64:
-// columns >= R are zero-filled by the TMA, which also cancels whatever follows dt in the x_proj rows).  The block's 128
-// weight rows (64 forward channels, 64 reverse) stay in shared memory for its whole life as the A operand; per chunk ONE
-// thread issues  D[128 x 32] = W[128 x 64] . dt_tile[32 x 64]^T  (tcgen05.mma, M 128, N 32: 16 forward steps | 16
-// reverse-box rows; the cross terms are wasted, at 0.5 MFLOP per chunk nobody cares) into one of two 32-column TMEM
-// stages, one chunk ahead of the recurrence.  TMEM lane = thread: tcgen05.ld hands every thread the 16 raw delta values of
-// ITS (direction, channel) for the chunk straight into registers -- no shared-memory round trip, one LDS per step less --
-// and they are rounded to bf16 exactly where the GEMM would have rounded them.
 template <typename T, bool PRECISE, int MODE>
 __global__ void __launch_bounds__(kScanThreads, PRECISE ? 1 : (kScanCH == 64 ? PCAD_SCAN_MINBLOCKS64 : PCAD_SCAN_MINBLOCKS))
 biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__ CUtensorMap tm_df,
               const __grid_constant__ CUtensorMap tm_bcf, const __grid_constant__ CUtensorMap tm_ur,
               const __grid_constant__ CUtensorMap tm_dr, const __grid_constant__ CUtensorMap tm_bcr,
-              const __grid_constant__ CUtensorMap tm_wf, const __grid_constant__ CUtensorMap tm_wr, int dt_ksteps,
               const T* __restrict__ z, long long ldz, const float* __restrict__ A_f, const float* __restrict__ D_f,
               const float* __restrict__ bias_f, const float* __restrict__ A_r, const float* __restrict__ D_r,
               const float* __restrict__ bias_r, T* y, int L, int E, const float* __restrict__ h0, int Lrun) {
-  constexpr bool FUSEDT = MODE == kScanFusedDt, BCF32 = MODE == kScanBcF32;
+  constexpr bool BCF32 = MODE == kScanBcF32;
   static_assert(MODE == kScanPlain || (sizeof(T) == 2 && !PRECISE && kScanCH == 64 && kScanTC == 16),
-                "the in-kernel dt_proj and the fp32 B|C rows are bf16-path features of the 64-channel, 16-step kernel");
-  // 1024-byte alignment: the swizzled tiles (TMA destinations, MMA operands) need it; the shared window of a CTA starts at
-  // an aligned address, so the declared alignment is the real one (checked below in the FUSEDT kernel)
+                "the fp32 B|C rows are a bf16-path feature of the 64-channel, 16-step kernel");
+  // TMA destinations need 128-byte alignment; the declared 1024 also rounds the static shared memory up to whole KB (the
+  // 41 KB per 64-channel block counted above)
   extern __shared__ __align__(1024) uint8_t scan_smem_raw[];
   typedef ScanShared<T, MODE> Shared;
   typedef ScanStage<T, MODE> Stage;
@@ -281,9 +249,6 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
   // kScanBcF32: two buffers (chunk parity), so that a chunk's main loop never writes what the previous chunk's epilogue reads.
   __shared__ __align__(16) float ys_all[BCF32 ? 2 : 1][2][kScanTC][kScanCH];
   __shared__ __align__(8) uint64_t full_bar[2];
-  __shared__ __align__(8) uint64_t dt_bar[2];    // FUSEDT: the stage's dt tile has landed (what the MMA issuer waits for)
-  __shared__ __align__(8) uint64_t w_bar;        // FUSEDT: the weight rows have landed
-  __shared__ uint32_t tmem_slot;
 
   const int tid = threadIdx.x;
   const int dir = tid / kScanCH;          // warp-uniform: the first half of the warps runs forward, the second half reverse
@@ -298,75 +263,33 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
   const int nch = (Lrun + kScanTC - 1) / kScanTC;
   constexpr int VEC = 16 / sizeof(T);              // elements per 16-byte vector
   constexpr int SEGS = kScanCH / VEC;              // 16-byte segments per 128-channel row
-  constexpr uint32_t kDtBytes = sizeof(T) * 2 * kScanTC * kScanDtK;
-  constexpr uint32_t kStageBytes = FUSEDT ? sizeof(Stage) - kDtBytes + sizeof(T) * 2 * kScanTC * 2 * kScanN : sizeof(Stage);
 
   if (tid == 0) {
-    // FUSEDT: a stage is full when its u / B|C loads have landed AND the MMA that turns its dt tile into delta (TMEM) has
-    // completed: the tcgen05.commit is the barrier's second arrival, so the block waits once per chunk
-    mbar_init(&full_bar[0], FUSEDT ? 2 : 1);
-    mbar_init(&full_bar[1], FUSEDT ? 2 : 1);
-    if constexpr (FUSEDT) {
-      if (smem_u32(scan_smem_raw) & 1023u) __trap();
-      mbar_init(&dt_bar[0], 1);
-      mbar_init(&dt_bar[1], 1);
-      mbar_init(&w_bar, 1);
-      tma_prefetch_desc(&tm_wf); tma_prefetch_desc(&tm_wr);
-    }
+    mbar_init(&full_bar[0], 1);
+    mbar_init(&full_bar[1], 1);
     fence_mbar_init();
     tma_prefetch_desc(&tm_uf); tma_prefetch_desc(&tm_df); tma_prefetch_desc(&tm_bcf);
     tma_prefetch_desc(&tm_ur); tma_prefetch_desc(&tm_dr); tma_prefetch_desc(&tm_bcr);
   }
-  uint32_t tmem = 0;
-  if constexpr (FUSEDT) {
-    if (tid < 32) {
-      tmem_alloc<kScanTmemCols>(&tmem_slot);
-      tmem_relinquish();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    tmem = tmem_slot;
-  } else {
-    __syncthreads();
-  }
+  __syncthreads();
 
   // chunk c: forward rows 16c .. 16c+15, reverse rows L-16(c+1) .. L-16c-1 (box row 15-j = step j).  One thread.
   auto issue = [&](int c, int stage) {
     Stage& s = sm.st[stage];
     uint64_t* bar = &full_bar[stage];
-    mbar_arrive_expect_tx(bar, kStageBytes);
+    mbar_arrive_expect_tx(bar, sizeof(Stage));
     const int rf = c * kScanTC, rr = L - (c + 1) * kScanTC;
     tma_load_3d(&s.u[0][0][0], &tm_uf, bar, e0, rf, seq);
     tma_load_3d(&s.u[1][0][0], &tm_ur, bar, e0, rr, seq);
-    if constexpr (FUSEDT) {
-      tma_load_3d(&sm.bc_raw[0][0][0], &tm_bcf, bar, 0, rf, seq);
-      tma_load_3d(&sm.bc_raw[1][0][0], &tm_bcr, bar, 0, rr, seq);
-      mbar_arrive_expect_tx(&dt_bar[stage], kDtBytes);
-      tma_load_3d(&s.dt[0][0][0], &tm_df, &dt_bar[stage], 0, rf, seq);
-      tma_load_3d(&s.dt[1][0][0], &tm_dr, &dt_bar[stage], 0, rr, seq);
+    if constexpr (BCF32) {
+      tma_load_3d(&s.bc[0][0][0], &tm_bcf, bar, 0, rf, seq);
+      tma_load_3d(&s.bc[1][0][0], &tm_bcr, bar, 0, rr, seq);
     } else {
-      if constexpr (BCF32) {
-        tma_load_3d(&s.bc[0][0][0], &tm_bcf, bar, 0, rf, seq);
-        tma_load_3d(&s.bc[1][0][0], &tm_bcr, bar, 0, rr, seq);
-      } else {
-        tma_load_3d(&s.bc_raw[0][0][0], &tm_bcf, bar, 0, rf, seq);
-        tma_load_3d(&s.bc_raw[1][0][0], &tm_bcr, bar, 0, rr, seq);
-      }
-      tma_load_3d(&s.d[0][0][0], &tm_df, bar, e0, rf, seq);
-      tma_load_3d(&s.d[1][0][0], &tm_dr, bar, e0, rr, seq);
+      tma_load_3d(&s.bc_raw[0][0][0], &tm_bcf, bar, 0, rf, seq);
+      tma_load_3d(&s.bc_raw[1][0][0], &tm_bcr, bar, 0, rr, seq);
     }
-  };
-  // FUSEDT, one thread: delta of chunk c (its dt tile has landed in `stage`) -> TMEM columns [32 stage, 32 stage + 32)
-  auto issue_dt_mma = [&](int c, int stage) {
-    if constexpr (FUSEDT) {
-      mbar_wait_or_trap(&dt_bar[stage], (c >> 1) & 1);
-      tc_fence_after();
-      constexpr uint32_t idesc = make_idesc_bf16(128, 2 * kScanTC);
-      const uint64_t da = make_smem_desc_sw128(smem_u32(&sm.wdt[0][0][0]));
-      const uint64_t db = make_smem_desc_sw128(smem_u32(&sm.st[stage].dt[0][0][0]));
-      umma_bf16_ss_k64_commit(tmem + stage * 2 * kScanTC, da, db, idesc, dt_ksteps, &full_bar[stage]);
-    }
+    tma_load_3d(&s.d[0][0][0], &tm_df, bar, e0, rf, seq);
+    tma_load_3d(&s.d[1][0][0], &tm_dr, bar, e0, rr, seq);
   };
 
   ScanDir<PRECISE> S;
@@ -380,39 +303,23 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
   const float Dskip = active ? (dir ? D_r : D_f)[e] : 0.f;
   const float bscale = ScanDir<PRECISE>::b_scale();
 
-  if (tid < 32 && elect_one()) {
-    if constexpr (FUSEDT) {
-      mbar_arrive_expect_tx(&w_bar, sizeof(sm.wdt));
-      tma_load_3d(&sm.wdt[0][0][0], &tm_wf, &w_bar, 0, e0, 0);
-      tma_load_3d(&sm.wdt[1][0][0], &tm_wr, &w_bar, 0, e0, 0);
-    }
-    issue(0, 0);
-    if constexpr (FUSEDT) {
-      mbar_wait_or_trap(&w_bar, 0);
-      issue_dt_mma(0, 0);
-    }
-  }
-  if constexpr (FUSEDT) mbar_wait_or_trap(&w_bar, 0);   // every later MMA issuer has observed the weight tile's arrival
+  if (tid < 32 && elect_one()) issue(0, 0);
   bool prev_late = false;
   for (int c = 0; c < nch; ++c) {
     const int stage = c & 1;
-    // Issue work: TMA by warp 0, the dt_proj MMA by warp 2 (a different scheduler: every instruction of these paths is on the
-    // block's critical path to the next barrier).  Whole warp into the branch, then elect.sync: the compiler then knows a
-    // single lane issues and emits the TMA / MMA instructions back to back instead of one election loop per instruction.
-    const bool tma_warp = tid < 32, mma_warp = (tid >> 5) == 2;
+    // TMA issue by warp 0.  Whole warp into the branch, then elect.sync: the compiler then knows a single lane issues and
+    // emits the TMA instructions back to back instead of one election loop per instruction.
     // every thread is past the barrier that followed chunk c-1's main loop: stage^1 is free to be overwritten
-    if constexpr (!FUSEDT) {
-      if (tma_warp && c + 1 < nch) {
-        if (elect_one()) issue(c + 1, stage ^ 1);
-      }
+    if (tid < 32 && c + 1 < nch) {
+      if (elect_one()) issue(c + 1, stage ^ 1);
     }
     const Stage& s = sm.st[stage];
     const int i0 = c * kScanTC;
     const int nsteps = min(kScanTC, Lrun - i0);
     const bool has_final = (L - 1 - (i0 + nsteps - 1)) < i0 + nsteps;
-    // (the fused kernel's barriers depend on descriptors and byte counts of two more async engines: a mistake there must
-    // trap, not hang the GPU)
-    if constexpr (MODE != kScanPlain) mbar_wait_or_trap(&full_bar[stage], (c >> 1) & 1);
+    // (kScanBcF32: the stage's byte count includes the fp32 B|C rows of a second buffer, through tensor maps of their own:
+    // a mismatch there must trap, not hang the GPU)
+    if constexpr (BCF32) mbar_wait_or_trap(&full_bar[stage], (c >> 1) & 1);
     else mbar_wait(&full_bar[stage], (c >> 1) & 1);
     float (*ys)[kScanTC][kScanCH] = ys_all[BCF32 ? (c & 1) : 0];
     const bool late_chunk = (L - 1 - i0) < i0;   // every position of the chunk was parked in an earlier chunk
@@ -423,9 +330,7 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
       for (int gi = tid; gi < 2 * kScanTC * 2 * kScanN / 4; gi += kScanThreads) {   // 256 groups of 4 values
         const int dd = gi >> 7, r = gi & 127;
         const int j = r >> 3, k0 = (r & 7) * 4;
-        const T* src;
-        if constexpr (FUSEDT) src = &sm.bc_raw[dd][dd ? kScanTC - 1 - j : j][k0];
-        else src = &s.bc_raw[dd][dd ? kScanTC - 1 - j : j][k0];
+        const T* src = &s.bc_raw[dd][dd ? kScanTC - 1 - j : j][k0];
         float4 v;
         if constexpr (sizeof(T) == 2) {
           const uint2 raw = *reinterpret_cast<const uint2*>(src);
@@ -438,13 +343,6 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
         *reinterpret_cast<float4*>(&sm.bc[dd][j][k0]) = v;
       }
       __syncthreads();   // sm.bc is complete; chunk c-1's epilogue (its parked partials, its reads of ys / pz) is done
-      if constexpr (FUSEDT) {
-        // the single B|C landing buffer has been consumed: only now may the next chunk's loads go out (they still have this
-        // chunk's whole main loop to arrive)
-        if (tma_warp && c + 1 < nch) {
-          if (elect_one()) issue(c + 1, stage ^ 1);
-        }
-      }
     } else {
       // No conversion pass, and normally no barrier here: the stage holds fp32 rows, ys is double-buffered, and in the
       // block-uniform ("late") path every thread prefetches into the very pz items it reads back in the epilogue.  The one
@@ -487,10 +385,7 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
     }
     cp_async_commit();
 
-    if constexpr (FUSEDT) tc_fence_after();   // delta of the chunk is in TMEM (the wait on full_bar above covered the MMA)
-    // FUSEDT: tcgen05.ld is .sync.aligned -- every lane of a warp must execute it, so lanes (and whole warps) past E run the
-    // recurrence too, on the zeros the TMA filled in for them (E is a multiple of 64 in every model; this is for the op API)
-    if (active || FUSEDT) {
+    if (active) {
       const float* bcp;
       if constexpr (BCF32) bcp = &s.bc[dir][0][0];
       else bcp = &sm.bc[dir][0][0];
@@ -513,86 +408,30 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
           dl = dl_n;
           return yv;
         };
-        if constexpr (FUSEDT) {
-          // this thread's TMEM lane holds delta of its channel: columns 0..15 forward steps, 16..31 the reverse box's rows
-          // (step j = row 15 - j).  Kept as 8 bf16 pairs in STEP order: pair q = steps 2q (low half), 2q + 1 (high half).
-          const uint32_t tmem_dl = tmem + (static_cast<uint32_t>((tid >> 5) * 32) << 16) + stage * 2 * kScanTC + (REV ? kScanTC : 0);
-          uint32_t dp2[kScanTC / 2 + 1];
-          {
-            uint32_t dr[kScanTC];
-            tmem_ld_32x32b_x16(tmem_dl, dr);
-            tmem_ld_wait();
-#pragma unroll
-            for (int q = 0; q < kScanTC / 2; ++q) {
-              const int c0 = REV ? kScanTC - 1 - 2 * q : 2 * q, c1 = REV ? kScanTC - 2 - 2 * q : 2 * q + 1;
-              dp2[q] = pack_bf16x2(__uint_as_float(dr[c0]), __uint_as_float(dr[c1]));
-            }
-            dp2[kScanTC / 2] = 0u;
-          }
-          auto lo = [](uint32_t w) { return __uint_as_float(w << 16); };
-          auto hi = [](uint32_t w) { return __uint_as_float(w & 0xffff0000u); };
-          dl = S.delta(lo(dp2[0]));
-          int j = 0;
-          // blocks of kScanUnroll steps reading a 5-pair window that slides by 4 pairs per block: one loop body
-          uint32_t w[kScanUnroll / 2 + 1];
-#pragma unroll
-          for (int q = 0; q <= kScanUnroll / 2; ++q) w[q] = dp2[q];
-          static_assert(kScanUnroll == 8, "the window logic below is written for 8-step blocks");
+        const T* dp = &s.d[REV ? 1 : 0][0][ch];
+        dl = S.delta(ActT<T>::to_f(dp[row(0)]));
+        // blocks of kScanUnroll steps with the stores deferred to the end of the block: no shared-memory store sits
+        // between the loads of consecutive steps, so the scheduler overlaps one step's tail with the next step's head
+        int j = 0;
 #pragma unroll 1
-          for (; j + kScanUnroll <= nsteps; j += kScanUnroll) {
-            float yv[kScanUnroll];
+        for (; j + kScanUnroll <= nsteps; j += kScanUnroll) {
+          float yv[kScanUnroll];
 #pragma unroll
-            for (int k = 0; k < kScanUnroll; ++k) {
-              const uint32_t wn = w[(k + 1) >> 1];
-              yv[k] = advance(j + k, min(j + k + 1, kScanTC - 1), ((k + 1) & 1) ? hi(wn) : lo(wn));
-            }
-#pragma unroll
-            for (int k = 0; k < kScanUnroll; ++k) ysp[(j + k) * kScanCH] = yv[k];
-#pragma unroll
-            for (int q = 0; q <= kScanUnroll / 2; ++q) w[q] = dp2[min(q + kScanUnroll / 2, kScanTC / 2)];
+          for (int k = 0; k < kScanUnroll; ++k) {
+            const int jn = min(j + k + 1, kScanTC - 1);
+            yv[k] = advance(j + k, jn, ActT<T>::to_f(dp[row(jn)]));
           }
-          // ragged last chunk: single steps, the next raw value re-read from TMEM (a dynamic column is an address there)
+#pragma unroll
+          for (int k = 0; k < kScanUnroll; ++k) ysp[(j + k) * kScanCH] = yv[k];
+        }
 #pragma unroll 1
-          for (; j < nsteps; ++j) {
-            const int jn = min(j + 1, kScanTC - 1);
-            const uint32_t rn = tmem_ld_32x32b_x1(tmem_dl + (REV ? kScanTC - 1 - jn : jn));
-            tmem_ld_wait();
-            ysp[j * kScanCH] = advance(j, jn, lo(pack_bf16x2(__uint_as_float(rn), 0.f)));
-          }
-        } else {
-          const T* dp = &s.d[REV ? 1 : 0][0][ch];
-          dl = S.delta(ActT<T>::to_f(dp[row(0)]));
-          // blocks of kScanUnroll steps with the stores deferred to the end of the block: no shared-memory store sits
-          // between the loads of consecutive steps, so the scheduler overlaps one step's tail with the next step's head
-          int j = 0;
-#pragma unroll 1
-          for (; j + kScanUnroll <= nsteps; j += kScanUnroll) {
-            float yv[kScanUnroll];
-#pragma unroll
-            for (int k = 0; k < kScanUnroll; ++k) {
-              const int jn = min(j + k + 1, kScanTC - 1);
-              yv[k] = advance(j + k, jn, ActT<T>::to_f(dp[row(jn)]));
-            }
-#pragma unroll
-            for (int k = 0; k < kScanUnroll; ++k) ysp[(j + k) * kScanCH] = yv[k];
-          }
-#pragma unroll 1
-          for (; j < nsteps; ++j) {
-            const int jn = min(j + 1, kScanTC - 1);
-            ysp[j * kScanCH] = advance(j, jn, ActT<T>::to_f(dp[row(jn)]));
-          }
+        for (; j < nsteps; ++j) {
+          const int jn = min(j + 1, kScanTC - 1);
+          ysp[j * kScanCH] = advance(j, jn, ActT<T>::to_f(dp[row(jn)]));
         }
       };
       if (dir) run_chunk(IntTag<1>());
       else run_chunk(IntTag<0>());
-    }
-    if constexpr (FUSEDT) {
-      tc_fence_before();   // this chunk's TMEM reads are ordered before the barrier below (the stage is rewritten two MMAs on)
-      // next chunk's delta: its dt tile was requested a whole main loop ago; the TMEM stage it writes was last read in
-      // chunk c-1, behind two block barriers
-      if (mma_warp && c + 1 < nch) {
-        if (elect_one()) issue_dt_mma(c + 1, stage ^ 1);
-      }
     }
     cp_async_wait<0>();
     __syncthreads();   // both directions' un-gated outputs of the chunk are in ys, partials / z in sm.pz
@@ -681,11 +520,6 @@ biscan_kernel(const __grid_constant__ CUtensorMap tm_uf, const __grid_constant__
     // no barrier here: the next iteration's first __syncthreads orders these reads of sm.ys and of the stage
     // against their next writers
   }
-  if constexpr (FUSEDT) {
-    tc_fence_before();
-    __syncthreads();
-    if (tid < 32) tmem_dealloc<kScanTmemCols>(tmem);
-  }
 }
 
 // B|C columns of the two x_proj outputs ([rows, ldbc] bf16, B at bc_off, C at bc_off + 16) -> float [2][rows][32] rows
@@ -710,37 +544,26 @@ __global__ void bc_to_f32_kernel(const bf16* __restrict__ dbc_f, const bf16* __r
   op[1] = o1;
 }
 
-// FUSEDT = true: delta_f / delta_r are the x_proj outputs ([S*L, ldbc], dt in columns 0..R-1, ldbc >= 64) and wdt_f / wdt_r
-// the dt_proj weights [E, R] (row pitch ldw, a multiple of 8 elements; R <= 64); otherwise delta_* are [S*L, E] and wdt_* unused.
+// u_* and delta_* are [S*L, E]; bc_* hold B|C at column bc_off of [S*L, ldbc] rows (read by kScanPlain, while kScanBcF32
+// reads bcf_*).  h0: the states each sequence starts from (time-parallel segments), or null for zeros.
 template <typename T, bool PRECISE, int MODE = kScanPlain>
 inline cudaError_t launch_biscan(const T* u_f, const T* delta_f, const T* bc_f, const T* u_r, const T* delta_r,
                                  const T* bc_r, long long ldbc, int bc_off, const T* z, long long ldz,
                                  const float* A_f, const float* D_f, const float* bias_f, const float* A_r,
                                  const float* D_r, const float* bias_r, T* y, int S, int L, int E,
-                                 cudaStream_t stream, const T* wdt_f = nullptr, const T* wdt_r = nullptr, long long ldw = 0,
-                                 int R = 0, const float* h0 = nullptr, int Lrun = 0, const float* bcf_f = nullptr,
+                                 cudaStream_t stream, const float* h0 = nullptr, int Lrun = 0, const float* bcf_f = nullptr,
                                  const float* bcf_r = nullptr) {
-  constexpr bool FUSEDT = MODE == kScanFusedDt, BCF32 = MODE == kScanBcF32;
+  constexpr bool BCF32 = MODE == kScanBcF32;
   size_t smem = sizeof(ScanShared<T, MODE>);
   if (const char* ex = getenv("PCAD_SCAN_EXTRA_SMEM")) smem += static_cast<size_t>(atoi(ex));   // occupancy experiments
   static unsigned long long attr_done = 0;
   cudaError_t e1 = ensure_dynamic_smem(biscan_kernel<T, PRECISE, MODE>, static_cast<int>(smem), attr_done);
   if (e1 != cudaSuccess) return e1;
   constexpr bool f32 = sizeof(T) == 4;
-  CUtensorMap tm[8];
+  CUtensorMap tm[6];
   bool ok = make_tmap_3d(&tm[0], f32, u_f, E, L, S, E, kScanCH, kScanTC) && make_tmap_3d(&tm[2], f32, u_r, E, L, S, E, kScanCH, kScanTC);
-  if (FUSEDT) {
-    if (ldbc < kScanDtK || !wdt_f || !wdt_r || R <= 0 || R > kScanDtK || ldw < R || (ldw % 8)) return cudaErrorInvalidValue;
-    ok = ok && make_tmap_3d(&tm[1], f32, delta_f, ldbc, L, S, ldbc, kScanDtK, kScanTC, true) &&
-         make_tmap_3d(&tm[3], f32, delta_r, ldbc, L, S, ldbc, kScanDtK, kScanTC, true);
-    ok = ok && make_tmap_3d(&tm[6], f32, wdt_f, R, E, 1, ldw, kScanDtK, kScanCH, true) &&
-         make_tmap_3d(&tm[7], f32, wdt_r, R, E, 1, ldw, kScanDtK, kScanCH, true);
-  } else {
-    ok = ok && make_tmap_3d(&tm[1], f32, delta_f, E, L, S, E, kScanCH, kScanTC) &&
-         make_tmap_3d(&tm[3], f32, delta_r, E, L, S, E, kScanCH, kScanTC);
-    tm[6] = tm[0];
-    tm[7] = tm[0];
-  }
+  ok = ok && make_tmap_3d(&tm[1], f32, delta_f, E, L, S, E, kScanCH, kScanTC) &&
+       make_tmap_3d(&tm[3], f32, delta_r, E, L, S, E, kScanCH, kScanTC);
   if (BCF32) {   // bcf_*: float [S*L, 32] rows [B ln 2 | C] (bc_to_f32_kernel)
     if (!bcf_f || !bcf_r) return cudaErrorInvalidValue;
     ok = ok && make_tmap_3d(&tm[4], true, bcf_f, 2 * kScanN, L, S, 2 * kScanN, 2 * kScanN, kScanTC);
@@ -752,8 +575,8 @@ inline cudaError_t launch_biscan(const T* u_f, const T* delta_f, const T* bc_f, 
   if (!ok) return cudaErrorInvalidValue;
   dim3 grid((E + kScanCH - 1) / kScanCH, S);
   biscan_kernel<T, PRECISE, MODE><<<grid, kScanThreads, smem, stream>>>(
-      tm[0], tm[1], tm[4], tm[2], tm[3], tm[5], tm[6], tm[7], (R + 15) / 16, z, ldz, A_f, D_f, bias_f, A_r, D_r, bias_r, y, L, E,
-      h0, (Lrun > 0 && Lrun < L) ? Lrun : L);
+      tm[0], tm[1], tm[4], tm[2], tm[3], tm[5], z, ldz, A_f, D_f, bias_f, A_r, D_r, bias_r, y, L, E, h0,
+      (Lrun > 0 && Lrun < L) ? Lrun : L);
   return cudaGetLastError();
 }
 
@@ -876,10 +699,10 @@ inline cudaError_t launch_biscan_time_parallel(const T* u_f, const T* delta_f, c
   if constexpr (sizeof(T) == 2 && !PRECISE) {
     if (bcf_f && bcf_r)
       return launch_biscan<T, PRECISE, kScanBcF32>(u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, bias_f, A_r,
-                                                   D_r, bias_r, y, S * P, Lseg, E, stream, nullptr, nullptr, 0, 0, state, 0, bcf_f, bcf_r);
+                                                   D_r, bias_r, y, S * P, Lseg, E, stream, state, 0, bcf_f, bcf_r);
   }
   return launch_biscan<T, PRECISE, kScanPlain>(u_f, delta_f, bc_f, u_r, delta_r, bc_r, ldbc, bc_off, z, ldz, A_f, D_f, bias_f, A_r, D_r,
-                                               bias_r, y, S * P, Lseg, E, stream, nullptr, nullptr, 0, 0, state);
+                                               bias_r, y, S * P, Lseg, E, stream, state);
 }
 
 }  // namespace pcad

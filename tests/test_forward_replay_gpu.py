@@ -36,7 +36,7 @@ RAGGED = (13, 301)           # T = 7826: ragged row and time tiles, below the fp
 SNP = (256, 512)             # bench.py --workload snp
 LONG = (16, 8192)            # bench.py --workload long
 BC_ROWS_MIN_T = 65536        # run_mixer_m1: fp32 B|C rows from this many rows on (bf16)
-SWITCHES = ("PCAD_SCAN_BC_F32", "PCAD_NO_PRUNE", "PCAD_NO_TIME_PARALLEL", "PCAD_FUSED_DT", "PCAD_NO_FUSED_NORM", "PCAD_SSD_SEQ")
+SWITCHES = ("PCAD_SCAN_BC_F32", "PCAD_NO_PRUNE", "PCAD_NO_TIME_PARALLEL", "PCAD_NO_FUSED_NORM", "PCAD_SSD_SEQ")
 
 
 # ---- the plan: modes the forward picks from the shape ------------------------------------------------------------------
