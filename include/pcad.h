@@ -94,7 +94,8 @@ int pcad_set_tokenizer(pcad_handle* h, const uint8_t lut[256], int mask_id, cons
 /* Replaces: model(input_ids=ids[, output_hidden_states=True])  (zero_shot_score.py:115,
  * train_XGBoost.py:104).  ids_dev: int64 [B, L] on the device.  logits_dev: float32 [B, L, V] or
  * NULL.  hidden_dev: [B, L, 2*d_model] in the model dtype (final normed hidden state,
- * hidden_states[-1]) or NULL. */
+ * hidden_states[-1]) or NULL: pcad_forward_taps with tap_idx = {n_layer}, bit-identical and with the same launches.
+ * Runs the whole model even when both outputs are NULL. */
 int pcad_forward(pcad_handle* h, const int64_t* ids_dev, int B, int L,
                  float* logits_dev, void* hidden_dev, void* stream);
 
@@ -114,7 +115,8 @@ int pcad_score_masked_at(pcad_handle* h, const uint8_t* ids_dev, int token_idx, 
 /* Replaces: model(input_ids, output_hidden_states=True).hidden_states[-1][:, tokenIdx, :]  (extract_embeddings,
  * train_XGBoost.py:104-105) without materialising [B, L, 2*d_model]: ids_dev uint8 [B, L] (masked or not, as the caller
  * wants), pos_dev int32 [B, n_pos]; hidden_dev receives [B, n_pos, 2*d_model] in the model dtype (forward half, then the
- * RC half with its channels in the reference's order -- the caller's `reverse[..., ::-1]` average applies as is). */
+ * RC half with its channels in the reference's order -- the caller's `reverse[..., ::-1]` average applies as is).
+ * pcad_hidden_at_layers with tap_idx = {n_layer}, bit-identical and with the same launches. */
 int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos,
                    void* hidden_dev, void* stream);
 
@@ -124,6 +126,7 @@ int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_de
  *   k = 0                the RCPS embedding;
  *   k in [1, n_layer)    layer k-1's mixer output: out_proj's result before the residual add, the tensor layer k receives;
  *   k = n_layer          the final normed state (pcad_forward's hidden_dev).
+ * With n_layer = 0 the tuple's one entry, k = 0, is the final normed state, written once.
  * tap_idx: n_taps host int32 indices, strictly increasing, in [0, n_layer]; tap_dev: host array of n_taps device pointers,
  * tap i receives hidden_states[tap_idx[i]].  The ids are checked as pcad_forward checks them.  Taps change no other output
  * bit: logits and every tap equal those of a call that requests any other set of taps, or none.  With logits_dev NULL the

@@ -612,8 +612,9 @@ __global__ void gather_rows_kernel(const uint4* __restrict__ src, uint4* __restr
 
 // ---- hidden-state taps ---------------------------------------------------------------------------------
 // Which entries of the reference's hidden_states tuple a forward emits, and where: idx[i] (strictly increasing, in
-// [0, n_layer]) goes to dst[i], [B, L, 2d] in the model dtype; or, with pos, [B, n_pos, 2d] at the positions pos[b, :];
-// or, with mean, float [B, 2d] at mean + i * B * 2d: the mean over each window's range (op_hidden_mean).
+// [0, n_layer]) goes to dst[i], [B, L, 2d] in the model dtype; or, with pos, [B, n_pos, 2d] at the positions pos[b, :],
+// at dst[0] + i * B * n_pos * 2d; or, with mean, float [B, 2d] at mean + i * B * 2d: the mean over each window's range
+// (op_hidden_mean).
 struct Taps {
   int n = 0;
   const int32_t* idx = nullptr;
@@ -646,8 +647,9 @@ int emit_tap(pcad_handle* h, const Taps* taps, int k, const void* src, int B, in
   if (taps->pos) {
     const long long total = static_cast<long long>(B) * taps->n_pos * (2 * d / 8);
     const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
-    if (h->f32) hidden_tap_pos_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(src), taps->pos, taps->n_pos, static_cast<float*>(taps->dst[i]), B, L, d);
-    else hidden_tap_pos_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(src), taps->pos, taps->n_pos, static_cast<bf16*>(taps->dst[i]), B, L, d);
+    void* dst = static_cast<uint8_t*>(taps->dst[0]) + static_cast<size_t>(i) * B * taps->n_pos * 2 * d * h->act_size;
+    if (h->f32) hidden_tap_pos_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(src), taps->pos, taps->n_pos, static_cast<float*>(dst), B, L, d);
+    else hidden_tap_pos_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(src), taps->pos, taps->n_pos, static_cast<bf16*>(dst), B, L, d);
   } else {
     const long long total = static_cast<long long>(B) * L * (2 * d / 8);
     const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
@@ -698,9 +700,10 @@ int run_backbone(pcad_handle* h, int B, int L, cudaStream_t st, int prune_idx = 
     if (fused) row_sumsq_kernel<<<static_cast<unsigned>((T + 7) / 8), 256, 0, st>>>(static_cast<const bf16*>(ws.resid), ws.sumsq[cur], T, d, parts);
     CUDA_TRY(h, cudaGetLastError());
   }
-  int rc = emit_tap(h, taps, 0, x, B, L, st);
-  if (rc) return rc;
   const int n_layer = h->cfg.n_layer;
+  // with n_layer = 0, index 0 is not the embedding but the final norm, emitted after it
+  int rc = n_layer > 0 ? emit_tap(h, taps, 0, x, B, L, st) : PCAD_OK;
+  if (rc) return rc;
   const int n_run = full || !taps ? n_layer : (taps->deepest() < n_layer ? taps->deepest() : n_layer);
   for (int li = 0; li < n_run; ++li) {
     LayerWeights& lw = h->layers[li];
@@ -840,8 +843,10 @@ int stage_ids64(pcad_handle* h, const int64_t* ids_dev, int B, int L, cudaStream
   return PCAD_OK;
 }
 
-// The tap list of pcad_forward_taps / pcad_hidden_at_layers, checked before anything is launched.
+// The handle and the tap list of pcad_forward_taps / pcad_hidden_at_layers / pcad_hidden_mean_at_layers, checked before
+// anything is launched.
 int check_taps(pcad_handle* h, int n_taps, const int32_t* tap_idx) {
+  if (!h) return PCAD_ERR_INVALID;
   const int n_layer = h->cfg.n_layer;
   if (n_taps < 1 || n_taps > n_layer + 1) return fail(h, PCAD_ERR_INVALID, "n_taps = %d outside [1, n_layer + 1 = %d]", n_taps, n_layer + 1);
   if (!tap_idx) return fail(h, PCAD_ERR_INVALID, "tap_idx is null");
@@ -850,6 +855,22 @@ int check_taps(pcad_handle* h, int n_taps, const int32_t* tap_idx) {
     if (i > 0 && tap_idx[i] <= tap_idx[i - 1]) return fail(h, PCAD_ERR_INVALID, "tap_idx is not strictly increasing at %d", i);
   }
   return PCAD_OK;
+}
+
+// The body of every entry point that writes hidden_states entries, after the entry's own checks: begin_call (count,
+// args_ok and args_msg as there; an empty call returns PCAD_OK), the ids staged from int64 ids64 or else from u8 ids8, the
+// backbone emitting `taps` (nullptr: none), then the head into logits_dev.  Without logits the backbone stops at the
+// deepest requested entry.
+int tapped_forward(pcad_handle* h, const int64_t* ids64, const uint8_t* ids8, int B, int L, int count, bool args_ok,
+                   const char* args_msg, const Taps* taps, float* logits_dev, void* stream) {
+  int rc = begin_call(h, B, L, count, args_ok, args_msg);
+  if (rc) return rc == kNoWork ? PCAD_OK : rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = ids64 ? stage_ids64(h, ids64, B, L, st) : stage_ids(h, ids8, B, L, -1, st);
+  if (rc) return rc;
+  rc = run_backbone(h, B, L, st, -1, taps, logits_dev != nullptr);
+  if (rc || !logits_dev) return rc;
+  return run_head(h, B, L, nullptr, 0, logits_dev, st);
 }
 
 // Backbone + head at token_idx -> out [B, 4]; ws.ids, ws.pos and ws.pos0 are staged.  One scored position, the same in every
@@ -1299,26 +1320,10 @@ int pcad_score_windows_dev(pcad_handle* h, const uint8_t* ascii_dev, int B, int 
 }
 
 int pcad_forward(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* logits_dev, void* hidden_dev, void* stream) {
-  int rc = begin_call(h, B, L, 1, ids_dev, "ids_dev is null");
-  if (rc) return rc == kNoWork ? PCAD_OK : rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = stage_ids64(h, ids_dev, B, L, st);
-  if (rc) return rc;
-  rc = run_backbone(h, B, L, st);
-  if (rc) return rc;
-  if (logits_dev) {
-    rc = run_head(h, B, L, nullptr, 0, logits_dev, st);
-    if (rc) return rc;
-  }
-  if (hidden_dev) {
-    StageTimer tm(h, st, PCAD_ST_MISC);
-    const long long total = static_cast<long long>(B) * L * (2 * h->d / 8);
-    const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
-    if (h->f32) hidden_tap_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(h->ws.normed), static_cast<float*>(hidden_dev), B, L, h->d);
-    else hidden_tap_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(h->ws.normed), static_cast<bf16*>(hidden_dev), B, L, h->d);
-    CUDA_TRY(h, cudaGetLastError());
-  }
-  return PCAD_OK;
+  if (!h) return PCAD_ERR_INVALID;
+  const int32_t last = h->cfg.n_layer;
+  Taps taps{1, &last, &hidden_dev};
+  return tapped_forward(h, ids_dev, nullptr, B, L, 1, ids_dev, "ids_dev is null", hidden_dev ? &taps : nullptr, logits_dev, stream);
 }
 
 int pcad_score_masked(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_mask, float* logits4_dev, void* stream) {
@@ -1342,85 +1347,43 @@ int pcad_score_masked_at(pcad_handle* h, const uint8_t* ids_dev, int token_idx, 
 }
 
 int pcad_hidden_at(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos, void* hidden_dev, void* stream) {
-  int rc = begin_call(h, B, L, n_pos, ids_dev && pos_dev && hidden_dev && n_pos >= 0, "null or negative argument");
-  if (rc) return rc == kNoWork ? PCAD_OK : rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = stage_ids(h, ids_dev, B, L, -1, st);
-  if (rc) return rc;
-  rc = run_backbone(h, B, L, st);
-  if (rc) return rc;
-  StageTimer tm(h, st, PCAD_ST_MISC);
-  const long long total = static_cast<long long>(B) * n_pos * (2 * h->d / 8);
-  const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
-  if (h->f32) hidden_tap_pos_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(h->ws.normed), pos_dev, n_pos, static_cast<float*>(hidden_dev), B, L, h->d);
-  else hidden_tap_pos_kernel<bf16><<<blocks, 256, 0, st>>>(static_cast<const bf16*>(h->ws.normed), pos_dev, n_pos, static_cast<bf16*>(hidden_dev), B, L, h->d);
-  CUDA_TRY(h, cudaGetLastError());
-  return PCAD_OK;
+  if (!h) return PCAD_ERR_INVALID;
+  const int32_t last = h->cfg.n_layer;
+  Taps taps{1, &last, &hidden_dev, pos_dev, n_pos};
+  return tapped_forward(h, nullptr, ids_dev, B, L, n_pos, ids_dev && pos_dev && hidden_dev && n_pos >= 0, "null or negative argument",
+                        &taps, nullptr, stream);
 }
 
 int pcad_forward_taps(pcad_handle* h, const int64_t* ids_dev, int B, int L, float* logits_dev, int n_taps, const int32_t* tap_idx,
                       void* const* tap_dev, void* stream) {
-  if (!h) return PCAD_ERR_INVALID;
   int rc = check_taps(h, n_taps, tap_idx);
   if (rc) return rc;
   if (!tap_dev) return fail(h, PCAD_ERR_INVALID, "tap_dev is null");
   for (int i = 0; i < n_taps; ++i)
     if (!tap_dev[i]) return fail(h, PCAD_ERR_INVALID, "tap_dev[%d] is null", i);
-  rc = begin_call(h, B, L, 1, ids_dev, "ids_dev is null");
-  if (rc) return rc == kNoWork ? PCAD_OK : rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = stage_ids64(h, ids_dev, B, L, st);
-  if (rc) return rc;
-  Taps taps;
-  taps.n = n_taps;
-  taps.idx = tap_idx;
-  taps.dst = tap_dev;
-  rc = run_backbone(h, B, L, st, -1, &taps, logits_dev != nullptr);
-  if (rc || !logits_dev) return rc;
-  return run_head(h, B, L, nullptr, 0, logits_dev, st);
+  Taps taps{n_taps, tap_idx, tap_dev};
+  return tapped_forward(h, ids_dev, nullptr, B, L, 1, ids_dev, "ids_dev is null", &taps, logits_dev, stream);
 }
 
 int pcad_hidden_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* pos_dev, int B, int L, int n_pos, int n_taps,
                           const int32_t* tap_idx, void* hidden_dev, void* stream) {
-  if (!h) return PCAD_ERR_INVALID;
   int rc = check_taps(h, n_taps, tap_idx);
   if (rc) return rc;
   if (!hidden_dev) return fail(h, PCAD_ERR_INVALID, "hidden_dev is null");
-  rc = begin_call(h, B, L, n_pos, ids_dev && pos_dev && n_pos >= 0, "null or negative argument");
-  if (rc) return rc == kNoWork ? PCAD_OK : rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = stage_ids(h, ids_dev, B, L, -1, st);
-  if (rc) return rc;
-  // tap i occupies [B, n_pos, 2d] of hidden_dev, after the i taps before it
-  const size_t tap_bytes = static_cast<size_t>(B) * n_pos * 2 * h->d * h->act_size;
-  std::vector<void*> dst(n_taps);
-  for (int i = 0; i < n_taps; ++i) dst[i] = static_cast<uint8_t*>(hidden_dev) + i * tap_bytes;
-  Taps taps;
-  taps.n = n_taps;
-  taps.idx = tap_idx;
-  taps.dst = dst.data();
-  taps.pos = pos_dev;
-  taps.n_pos = n_pos;
-  return run_backbone(h, B, L, st, -1, &taps, false);
+  Taps taps{n_taps, tap_idx, &hidden_dev, pos_dev, n_pos};
+  return tapped_forward(h, nullptr, ids_dev, B, L, n_pos, ids_dev && pos_dev && n_pos >= 0, "null or negative argument", &taps,
+                        nullptr, stream);
 }
 
 int pcad_hidden_mean_at_layers(pcad_handle* h, const uint8_t* ids_dev, const int32_t* ranges_dev, int B, int L, int n_taps,
                                const int32_t* tap_idx, float* out_dev, void* stream) {
-  if (!h) return PCAD_ERR_INVALID;
   int rc = check_taps(h, n_taps, tap_idx);
   if (rc) return rc;
   if (!out_dev) return fail(h, PCAD_ERR_INVALID, "out_dev is null");
-  rc = begin_call(h, B, L, 1, ids_dev != nullptr, "ids_dev is null");
-  if (rc) return rc == kNoWork ? PCAD_OK : rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = stage_ids(h, ids_dev, B, L, -1, st);
-  if (rc) return rc;
-  Taps taps;
-  taps.n = n_taps;
-  taps.idx = tap_idx;
+  Taps taps{n_taps, tap_idx};
   taps.mean = out_dev;
   taps.ranges = ranges_dev;
-  return run_backbone(h, B, L, st, -1, &taps, false);
+  return tapped_forward(h, nullptr, ids_dev, B, L, 1, ids_dev != nullptr, "ids_dev is null", &taps, nullptr, stream);
 }
 
 int pcad_score_windows_host(pcad_handle* h, const uint8_t* ascii_host, int B, int L, int token_idx, float* logits4_host, void* stream) {

@@ -3,9 +3,9 @@
 halves averaged as ``(fwd + rev[..., ::-1]) / 2``.  The XGBoost classifier around it is CPU post-processing and stays with
 the caller.
 
-The reference materialises ``hidden_states[-1]`` ([B, L, 2d]) to read one position; here ``pcad_hidden_at`` taps the
-requested position(s) only, windows travel as ASCII bytes and are tokenised with the byte LUT (the reference's dataset for
-this script does NOT mask ``tokenIdx``: the embedding is taken from the unmasked window).
+The reference materialises ``hidden_states[-1]`` ([B, L, 2d]) to read one position; here ``pcad_hidden_at_layers`` taps
+the requested position(s) only, windows travel as ASCII bytes and are tokenised with the byte LUT (the reference's dataset
+for this script does NOT mask ``tokenIdx``: the embedding is taken from the unmasked window).
 """
 from __future__ import annotations
 
@@ -46,10 +46,10 @@ def extract_embeddings(model, tokenizer, sequences: Union[Sequence[str], np.ndar
     if ranges is not None and pooling != "mean":
         raise ValueError("ranges apply to pooling='mean' only")
     many = not isinstance(layer, numbers.Integral) or isinstance(layer, bool)
-    if many:
-        layers = hidden_layer_indices(layer, model.config.n_layer)
-    else:
-        layers = None if int(layer) == -1 else hidden_layer_indices([layer], model.config.n_layer)   # -1: hidden_at's own path
+    layers = hidden_layer_indices(layer if many else [layer], model.config.n_layer)
+    # the final state, however it is spelled, is hidden_at's and hidden_mean's default: a model object that has only
+    # hidden_at(ids, pos) serves the reference's own call
+    kw = {} if layers == [model.config.n_layer] else {"layers": layers}
     if isinstance(sequences, np.ndarray):
         ascii_mat = np.ascontiguousarray(sequences, dtype=np.uint8)
     else:
@@ -57,20 +57,14 @@ def extract_embeddings(model, tokenizer, sequences: Union[Sequence[str], np.ndar
         ascii_mat = tokenizer.windows_to_ascii(seqs, len(seqs[0])) if seqs else np.zeros((0, 0), dtype=np.uint8)
     n = len(ascii_mat)
     rng = None if ranges is None else hidden_mean_ranges(ranges, n, ascii_mat.shape[1])
-    n_out = len(layers) if layers is not None else 1
-    out = np.zeros((n_out, n, 2 * model.config.d_model), dtype=np.float32)
+    out = np.zeros((len(layers), n, 2 * model.config.d_model), dtype=np.float32)
     for s in range(0, n, batch_size):
         ids = tokenizer.encode_bytes(ascii_mat[s:s + batch_size])
         if pooling == "mean":
             r = rng[s:s + len(ids)] if rng is not None else None
-            h = model.hidden_mean(torch.from_numpy(ids), r, layers=layers)
-            out[:, s:s + len(ids)] = (h[None] if layers is None else h).cpu().numpy()
-            continue
-        pos = torch.full((len(ids), 1), int(tokenIdx), dtype=torch.int32)
-        if layers is None:
-            h = model.hidden_at(torch.from_numpy(ids), pos)[None, :, 0]
+            h = model.hidden_mean(torch.from_numpy(ids), r, **kw)
         else:
-            h = model.hidden_at(torch.from_numpy(ids), pos, layers=layers)[:, :, 0]
-        out[:, s:s + len(ids)] = h.to(torch.float32).cpu().numpy()
+            h = model.hidden_at(torch.from_numpy(ids), torch.full((len(ids), 1), int(tokenIdx), dtype=torch.int32), **kw)
+        out[:, s:s + len(ids)] = h.to(torch.float32).reshape(len(layers), len(ids), -1).cpu().numpy()
     out = out if many else out[0]
     return average_strands(out) if average else out

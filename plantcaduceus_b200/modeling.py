@@ -258,45 +258,44 @@ class CaduceusForMaskedLM:
         self._require_handle()
         if input_ids is None or input_ids.dim() != 2:
             raise ValueError("input_ids must be a [batch, length] integer tensor")
-        if hidden_layers is not None:
-            return self._forward_taps(input_ids, hidden_layer_indices(hidden_layers, self.config.n_layer), compute_logits)
+        want, idx, _ = self._tap_indices(hidden_layers)
         ids = input_ids.to(device=self.device, dtype=torch.int64).contiguous()
         B, L = ids.shape
         with torch.cuda.device(self.device):
             logits = torch.empty((B, L, self.config.vocab_size), dtype=torch.float32, device=self.device) \
                 if compute_logits else None
-            hidden = torch.empty((B, L, 2 * self.config.d_model), dtype=self.dtype, device=self.device) \
-                if output_hidden_states else None
+            taps = [torch.empty((B, L, 2 * self.config.d_model), dtype=self.dtype, device=self.device) for _ in want] \
+                if output_hidden_states or hidden_layers is not None else []
             if B > 0 and L > 0:
-                _lib.check(self._lib.pcad_forward(
-                    self._handle, C.c_void_p(ids.data_ptr()), B, L,
-                    C.c_void_p(logits.data_ptr()) if logits is not None else None,
-                    C.c_void_p(hidden.data_ptr()) if hidden is not None else None, self._stream()), self._handle)
+                lg = C.c_void_p(logits.data_ptr()) if logits is not None else None
+                if hidden_layers is None:   # the C drop-in for model(ids): the launches of pcad_forward_taps([n_layer])
+                    _lib.check(self._lib.pcad_forward(self._handle, C.c_void_p(ids.data_ptr()), B, L, lg,
+                                                      C.c_void_p(taps[0].data_ptr()) if taps else None, self._stream()),
+                               self._handle)
+                else:
+                    ptrs = (C.c_void_p * len(want))(*[t.data_ptr() for t in taps])
+                    _lib.check(self._lib.pcad_forward_taps(self._handle, C.c_void_p(ids.data_ptr()), B, L, lg, len(want), idx,
+                                                           ptrs, self._stream()), self._handle)
                 self._raise_on_bad_ids(True)
-        # hidden_states: only the final (normed) state is materialised; hidden_states[-1] is what the
-        # reference's callers read (train_XGBoost.py:105, notebooks/examples.ipynb:183).
-        return MaskedLMOutput(logits=logits, hidden_states=(hidden,) if hidden is not None else None)
-
-    def _forward_taps(self, input_ids: torch.Tensor, layers: List[int], compute_logits: bool) -> MaskedLMOutput:
-        ids = input_ids.to(device=self.device, dtype=torch.int64).contiguous()
-        B, L = ids.shape
-        want = sorted(layers)
-        with torch.cuda.device(self.device):
-            logits = torch.empty((B, L, self.config.vocab_size), dtype=torch.float32, device=self.device) \
-                if compute_logits else None
-            taps = [torch.empty((B, L, 2 * self.config.d_model), dtype=self.dtype, device=self.device) for _ in want]
-            if B > 0 and L > 0:
-                idx = (C.c_int32 * len(want))(*want)
-                ptrs = (C.c_void_p * len(want))(*[t.data_ptr() for t in taps])
-                _lib.check(self._lib.pcad_forward_taps(
-                    self._handle, C.c_void_p(ids.data_ptr()), B, L,
-                    C.c_void_p(logits.data_ptr()) if logits is not None else None, len(want), idx, ptrs,
-                    self._stream()), self._handle)
-                self._raise_on_bad_ids(True)
+        if hidden_layers is None:
+            # hidden_states: only the final (normed) state is materialised; hidden_states[-1] is what the
+            # reference's callers read (train_XGBoost.py:105, notebooks/examples.ipynb:183).
+            return MaskedLMOutput(logits=logits, hidden_states=tuple(taps) or None)
         hidden: List[Optional[torch.Tensor]] = [None] * (self.config.n_layer + 1)
         for k, t in zip(want, taps):
             hidden[k] = t
         return MaskedLMOutput(logits=logits, hidden_states=tuple(hidden))
+
+    def _tap_indices(self, layers: Union[None, str, Iterable[int]]) -> Tuple[List[int], C.Array, Optional[List[int]]]:
+        """``layers`` as ``forward``'s ``hidden_layers`` (None: the final normed state) in the form the engine takes them:
+        (the indices in increasing order, the same as a ctypes int32 array, and the permutation that puts results stacked
+        in that order back into the caller's order, or None where the two orders agree).  Raises ValueError as
+        ``hidden_layer_indices``."""
+        n_layer = self.config.n_layer
+        layers = [n_layer] if layers is None else hidden_layer_indices(layers, n_layer)
+        want = sorted(layers)
+        back = None if want == layers else [want.index(k) for k in layers]
+        return want, (C.c_int32 * len(want))(*want), back
 
     def _raise_on_bad_ids(self, sync: bool):
         """Token ids outside [0, vocab_size) raise IndexError, as the reference's nn.Embedding lookup would
@@ -342,41 +341,23 @@ class CaduceusForMaskedLM:
         ``layers`` ("all", or indices into hidden_states as ``forward``'s ``hidden_layers``): [len(layers), B, n_pos,
         2*d_model], entry i from hidden_states[layers[i]]; the forward stops after the deepest requested layer."""
         self._require_handle()
-        if layers is not None:
-            return self._hidden_at_layers(ids_u8, positions, hidden_layer_indices(layers, self.config.n_layer))
+        want, idx, back = self._tap_indices(layers)
         ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
         pos = positions.to(device=self.device, dtype=torch.int32).contiguous()
         B, L = ids.shape
         if pos.dim() == 1:
             pos = pos[:, None]
         n_pos = pos.shape[1]
-        with torch.cuda.device(self.device):
-            out = torch.empty((B, n_pos, 2 * self.config.d_model), dtype=self.dtype, device=self.device)
-            if B > 0 and L > 0 and n_pos > 0:
-                _lib.check(self._lib.pcad_hidden_at(self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(pos.data_ptr()),
-                                                    B, L, n_pos, C.c_void_p(out.data_ptr()), self._stream()), self._handle)
-                self._raise_on_bad_ids(True)
-        return out
-
-    def _hidden_at_layers(self, ids_u8: torch.Tensor, positions: torch.Tensor, layers: List[int]) -> torch.Tensor:
-        ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
-        pos = positions.to(device=self.device, dtype=torch.int32).contiguous()
-        B, L = ids.shape
-        if pos.dim() == 1:
-            pos = pos[:, None]
-        n_pos = pos.shape[1]
-        want = sorted(layers)
         with torch.cuda.device(self.device):
             out = torch.empty((len(want), B, n_pos, 2 * self.config.d_model), dtype=self.dtype, device=self.device)
             if B > 0 and L > 0 and n_pos > 0:
-                idx = (C.c_int32 * len(want))(*want)
                 _lib.check(self._lib.pcad_hidden_at_layers(self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(pos.data_ptr()),
                                                            B, L, n_pos, len(want), idx, C.c_void_p(out.data_ptr()),
                                                            self._stream()), self._handle)
                 self._raise_on_bad_ids(True)
-            if want != layers:   # the engine takes the indices in increasing order; return them in the caller's
-                out = out[torch.tensor([want.index(k) for k in layers], device=self.device)]
-        return out
+            if back is not None:
+                out = out[back]
+        return out[0] if layers is None else out
 
     def hidden_mean(self, ids_u8: torch.Tensor, ranges=None, layers: Union[None, str, Iterable[int]] = None) -> torch.Tensor:
         """Mean over each window's positions of a ``hidden_states`` entry, float32, without [B, L, 2*d_model] buffers:
@@ -387,25 +368,22 @@ class CaduceusForMaskedLM:
         order.  The forward stops after the deepest requested layer.  Raises ValueError for ranges that are not [B, 2]
         integers."""
         self._require_handle()
-        final = layers is None
-        want_layers = [self.config.n_layer] if final else hidden_layer_indices(layers, self.config.n_layer)
+        want, idx, back = self._tap_indices(layers)
         ids = ids_u8.to(device=self.device, dtype=torch.uint8).contiguous()
         B, L = ids.shape
         rng = None if ranges is None else hidden_mean_ranges(ranges, B, L).to(self.device)
-        want = sorted(want_layers)
         with torch.cuda.device(self.device):
             out = torch.empty((len(want), B, 2 * self.config.d_model), dtype=torch.float32, device=self.device)
             if B > 0 and L > 0:
-                idx = (C.c_int32 * len(want))(*want)
                 _lib.check(self._lib.pcad_hidden_mean_at_layers(
                     self._handle, C.c_void_p(ids.data_ptr()), C.c_void_p(rng.data_ptr()) if rng is not None else None, B, L,
                     len(want), idx, C.c_void_p(out.data_ptr()), self._stream()), self._handle)
                 self._raise_on_bad_ids(True)
             else:
                 out.fill_(float("nan"))   # L = 0: no range is valid
-            if want != want_layers:   # the engine takes the indices in increasing order; return them in the caller's
-                out = out[torch.tensor([want.index(k) for k in want_layers], device=self.device)]
-        return out[0] if final else out
+            if back is not None:
+                out = out[back]
+        return out[0] if layers is None else out
 
     def score_windows_host(self, ascii_windows: Union[np.ndarray, torch.Tensor], token_idx: int,
                            out: Optional[torch.Tensor] = None) -> torch.Tensor:
